@@ -10,7 +10,7 @@ it the CUDA path) to the reference's own PyTorch modules:
   deltas), one weight-loop training step (NVFPCC.py:149-197) on 2 real
   synthetic leaf blocks incl. every parameter/embedding gradient.
 * nvf_B.npz  chanstr 16,32,16,16 ch=3: decode of 1 block.
-* nvf_train2.npz  two more weight-loop steps of the reference: config A at q=1
+* nvf_train2_A.npz / nvf_train2_B.npz  two more weight-loop steps of the reference: config A at q=1
   (the noisy-kernel phase the bench runs; the uniform noises the reference drew
   are stored so the step can be replayed exactly) and config B at q=2.
 
@@ -35,6 +35,9 @@ from nvfpcc_b200 import synth  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 TRAIN_HP = dict(lmbda=200.0, w1=10.0, w2=57.0)
+# intra-op threads of the generating run: the CPU convolutions split their sums by thread count, so the float32
+# outputs stored here are bit-exact only under this count (tests/test_oracle_golden.py runs the oracle with it)
+GOLDEN_THREADS = 8
 
 
 def perturbed_state(ch, channels, seed=1234):
@@ -141,8 +144,8 @@ def reference_train_step(net, RL, fx, gt, dist, q, seed, n_total=849338.0):
 
 
 def gen_train2(RL):
-    save = {}
     for tag, q, blocks, seed in (("A", 1, (0, 600), 777), ("B", 2, (300,), 778)):
+        save = {}
         fx = fixture_inputs(tag)
         net = ref_import.build_net(fx["ch"], fx["channels"])
         net.load_state_dict(fx["sd"], strict=True)
@@ -153,9 +156,9 @@ def gen_train2(RL):
         save[pre + "dist"] = dist.astype(np.float32)
         for k, v in r.items():
             save[pre + k] = v
-    path = os.path.join(GOLDEN, "nvf_train2.npz")
-    np.savez_compressed(path, **save)
-    print("wrote", path, os.path.getsize(path) // 1024, "KiB")
+        path = os.path.join(GOLDEN, "nvf_train2_%s.npz" % tag)        # one file per step: each stays under 1 MB
+        np.savez_compressed(path, **save)
+        print("wrote", path, os.path.getsize(path) // 1024, "KiB")
 
 
 def _load_into_reference(net, sd):
@@ -165,7 +168,7 @@ def _load_into_reference(net, sd):
 
 def main():
     os.makedirs(GOLDEN, exist_ok=True)
-    torch.set_num_threads(max(1, os.cpu_count() or 1))
+    torch.set_num_threads(GOLDEN_THREADS)
     _, RL, _ = ref_import.load()
     if "--train2-only" in sys.argv:
         return gen_train2(RL)

@@ -22,6 +22,18 @@ def eff_weights(sd, q, dev, grad=False):
 _FIELDS = ()
 
 
+def run_without_gpu(code):
+    """Runs `code` in a child Python that sees no CUDA device, from the repository root, so that what the package
+    does without a GPU is checked on a machine with one as well.  Fails when the child exits non-zero."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, "-c", code], cwd=root, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]
+
+
 def logit_of(p):
     p = p.double().clamp(1e-12, 1 - 1e-12)
     return torch.log(p) - torch.log1p(-p)

@@ -51,9 +51,9 @@ def test_workspace_query_needs_no_device():
 
 def test_product_path_has_no_cpu_fallback():
     """Calling the product ops without a GPU must fail loudly, never fall back."""
-    import torch
-    from nvfpcc_b200 import ops
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(RuntimeError):
-        ops.decode_blocks(3, (8, 16, 8, 8), {}, torch.zeros(1, 3, 2, 2, 2), None, 0.5)
+    from tests.helpers import run_without_gpu
+    run_without_gpu("import pytest, torch\n"
+                    "from nvfpcc_b200 import ops\n"
+                    "assert not torch.cuda.is_available()\n"
+                    "with pytest.raises(RuntimeError):\n"
+                    "    ops.decode_blocks(3, (8, 16, 8, 8), {}, torch.zeros(1, 3, 2, 2, 2), None, 0.5)\n")

@@ -20,7 +20,7 @@ N_TOTAL = 849338.0
 
 @pytest.fixture(scope="module")
 def golden_train2():
-    return np.load(os.path.join(GOLDEN, "nvf_train2.npz"))
+    return {tag: np.load(os.path.join(GOLDEN, "nvf_train2_%s.npz" % tag)) for tag in "AB"}
 
 
 def _net(tag, fx):
@@ -63,7 +63,7 @@ def test_reference_train_step_q1_A_and_q2_B(gpu, golden_train2, tag, q):
     """One weight-loop step (NVFPCC.py:149-197) of the UNMODIFIED reference modules, stored by oracle/gen_golden.py:
     config A at q=1 (noisy kernels: the phase bench.py times) and config B at q=2.  Probabilities within the 1e-4
     logit band, every loss term, every parameter gradient and d/d-emb."""
-    g, pre = golden_train2, "%sq%d_" % (tag, q)
+    g, pre = golden_train2[tag], "%sq%d_" % (tag, q)
     fx = fixture_inputs(tag)
     net = _net(tag, fx)
     emb = fx["emb"].clone().cuda().requires_grad_(True)

@@ -116,7 +116,7 @@ def test_fused_step_matches_reference_golden(gpu, tag, q):
     """nvf_train_step with the reference's own noise draws handed in, against the golden steps produced by the
     UNMODIFIED reference modules (oracle/gen_golden.py gen_train2): loss terms and every raw-parameter gradient."""
     from nvfpcc_b200 import trainer
-    g, pre = np.load(os.path.join(GOLDEN, "nvf_train2.npz")), "%sq%d_" % (tag, q)
+    g, pre = np.load(os.path.join(GOLDEN, "nvf_train2_%s.npz" % tag)), "%sq%d_" % (tag, q)
     fx = fixture_inputs(tag)
     net = _net(fx)
     gt, dist = torch.from_numpy(g[pre + "gt"]).float().cuda(), torch.from_numpy(g[pre + "dist"]).float().cuda()

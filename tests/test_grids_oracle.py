@@ -88,9 +88,9 @@ def test_prep_header_symbols_are_exported_and_bound():
 
 
 def test_grids_have_no_cpu_fallback():
-    import torch
-    from nvfpcc_b200 import grids
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(RuntimeError):
-        grids.build_grids(np.zeros((1, 3), np.int32), np.zeros((1, 3), np.int32))
+    from tests.helpers import run_without_gpu
+    run_without_gpu("import numpy as np, pytest, torch\n"
+                    "from nvfpcc_b200 import grids\n"
+                    "assert not torch.cuda.is_available()\n"
+                    "with pytest.raises(RuntimeError):\n"
+                    "    grids.build_grids(np.zeros((1, 3), np.int32), np.zeros((1, 3), np.int32))\n")

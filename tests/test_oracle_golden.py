@@ -5,7 +5,17 @@ import pytest
 import torch
 
 from oracle import nvf_oracle as O
-from oracle.gen_golden import TRAIN_HP, fixture_inputs, state_checksum
+from oracle.gen_golden import GOLDEN_THREADS, TRAIN_HP, fixture_inputs, state_checksum
+
+
+@pytest.fixture(autouse=True, scope="module")
+def golden_threads():
+    """The golden float32 outputs are bit-exact only under the summation order they were made with, and the CPU
+    convolutions split their work - and so their sums - by the number of threads: run the oracle with that count."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 @pytest.mark.parametrize("tag", ["A", "B"])
@@ -84,14 +94,14 @@ def test_threshold_points_order():
 def golden_train2():
     import os
     from tests.conftest import GOLDEN
-    return np.load(os.path.join(GOLDEN, "nvf_train2.npz"))
+    return {tag: np.load(os.path.join(GOLDEN, "nvf_train2_%s.npz" % tag)) for tag in "AB"}
 
 
 @pytest.mark.parametrize("tag,q", [("A", 1), ("B", 2)])
 def test_train_step_q1_A_and_q2_B_match_reference(golden_train2, tag, q):
     """The two extra reference steps (oracle/gen_golden.py gen_train2): config A in the noisy-kernel phase
     (q=1, the phase bench.py runs) with the reference's own uniform draws replayed, and config B at q=2."""
-    g, pre = golden_train2, "%sq%d_" % (tag, q)
+    g, pre = golden_train2[tag], "%sq%d_" % (tag, q)
     fx = fixture_inputs(tag)
     sd = {k: v.clone().requires_grad_(not (k.endswith("_init") or k.endswith("pedestal"))) for k, v in fx["sd"].items()}
     emb = fx["emb"].clone().requires_grad_(True)
