@@ -6,7 +6,6 @@
 #include <stdlib.h>
 #include "../../include/nvf_b200.h"
 #include "nvf_common.h"
-#include "nvf_decode_fused.h"
 #include "nvf_emit.h"
 #include "nvf_layers.h"
 
@@ -15,7 +14,6 @@ namespace nvf {
 constexpr int kMaxCtas = 160;  // upper bound on persistent CTAs (B200: 148 SMs)
 constexpr size_t kAlign = 256;
 inline size_t align_up(size_t v) { return (v + kAlign - 1) / kAlign * kAlign; }
-inline bool is_cfg_A(const NvfDesc& d) { return d.ch == 3 && d.c0 == 8 && d.c1 == 16 && d.c2 == 8 && d.c3 == 8; }
 constexpr int64_t kGenericDecodeChunk = 128;  // blocks per pass of the layer-wise decode path
 // per-leaf scratch of the two-pass (wide) head: conv2 rows next to the cut + their partial logits
 inline size_t head_brow_floats(const NvfDesc& d) { return d.c3 == 16 ? (size_t)2 * d.c3 * 1024 : 0; }
@@ -70,8 +68,6 @@ struct DecodeWs {
       o += align_up(sizeof(float) * head_brow_floats(d) * (size_t)chunk);
       L.off_pl = o;
       o += align_up(sizeof(float) * head_pl_floats(d) * (size_t)chunk);
-    } else if (is_cfg_A(d)) {
-      o += align_up(sizeof(float) * (size_t)FusedA::SCRATCH_FLOATS * kMaxCtas);
     } else {
       const int64_t chunk = n < kGenericDecodeChunk ? n : kGenericDecodeChunk;
       o += align_up(sizeof(float) * (size_t)(Stash::make(d).per_block + kVox) * (size_t)chunk);
@@ -86,7 +82,7 @@ struct DecodeWs {
 };
 
 struct TrainWs {
-  size_t off_packed, off_stash, off_grad, off_tmp3, off_tmp1, off_gl2, off_gl1, off_gl0, off_p2, off_p1, off_p0, off_loss, off_partial, off_queue, off_pad, total;
+  size_t off_packed, off_stash, off_grad, off_tmp3, off_tmp1, off_gl2, off_gl1, off_gl0, off_p2, off_p1, off_p0, off_loss, off_partial, off_queue, total;
   static TrainWs make(const NvfDesc& d, int64_t n) {
     TrainWs L{};
     const Stash s = Stash::make(d);
@@ -106,10 +102,6 @@ struct TrainWs {
     L.off_loss = take(sizeof(double) * (size_t)NVF_LOSS_SUMS * (n * kLossChunks + 1));
     L.off_partial = take(sizeof(float) * partial_floats(d, n));
     L.off_queue = take(2 * 16 * kQueueSlots);   // forward slots, then backward slots
-    {   // zero-padded copy of the input of a transposed conv (polyphase forward kernels): max over up1 / up2
-      const size_t p1 = (size_t)d.c1 * 8 * 12 * 16, p2 = (size_t)d.c2 * 16 * 20 * 24;
-      L.off_pad = take(sizeof(float) * (p1 > p2 ? p1 : p2) * n);
-    }
     L.total = o;
     return L;
   }
@@ -221,7 +213,7 @@ struct Api {
     }
     // up1: convT k5 s2 p0 + ReLU (:4693-4700, :4762)
     p = LayerParams{a1, a2, packed + g.up1, w.up1_b, nullptr, nullptr, n, d.c1, d.c2, 8, 8, 19, 20, 0, ACT_RELU, OP_CONVT};
-    // decode (many leaves): polyphase kernel on a zero-padded copy of conv0's output; else the tile kernels
+    // fused-head decode (pad_scratch): polyphase kernel on a zero-padded copy of conv0's output; else the tile kernels
     if (!(pad_scratch && l.up_poly(p, pad_scratch))) layer(l, p);
     // conv1: conv k4 + ReLU (:4702-4710, :4763)
     p = LayerParams{a2, a3, packed + g.conv1, w.conv1_b, nullptr, nullptr, n, d.c2, d.c2, 19, 20, 16, 16, 0, ACT_RELU, OP_CORR4};
@@ -239,7 +231,7 @@ struct Api {
     }
     // up2: convT k5 s2 p0 + ReLU (:4712-4719, :4765)
     p = LayerParams{a3, a4, packed + g.up2, w.up2_b, nullptr, nullptr, n, d.c2, d.c3, 16, 16, 35, 36, 0, ACT_RELU, OP_CONVT};
-    if (!(pad_scratch && l.up_poly(p, pad_scratch))) layer(l, p);
+    layer(l, p);
     // conv2: conv k4 + ReLU (:4721-4729, :4766)
     p = LayerParams{a4, a5, packed + g.conv2, w.conv2_b, nullptr, nullptr, n, d.c3, d.c3, 35, 36, 32, 32, 0, ACT_RELU, OP_CORR4};
     layer(l, p);
@@ -271,7 +263,7 @@ struct Api {
         const GenericPacked g = GenericPacked::make(*desc);
         pack_all(l, *desc, *w, packed, false, false);
         PackParams pp{};
-        pp.job[pp.njobs++] = PackJob{w->cls2_w, packed + g.fusedA, PACK_CLS_IS, 1, desc->c3, 3};
+        pp.job[pp.njobs++] = PackJob{w->cls2_w, packed + g.cls_is, PACK_CLS_IS, 1, desc->c3, 3};
         l.pack(pp);
         const int64_t chunk = head_chunk(*desc, n_blocks);
         float* stash = (float*)(ws + W.off_scratch);
@@ -282,38 +274,12 @@ struct Api {
           forward_layers(l, *desc, *w, packed, latent + b0 * desc->ch * 8, nb, stash, nullptr, nullptr, nullptr, nullptr,
                          nullptr, nullptr, true, sp);   // sp doubles as the padded conv0 output until conv1 is done
           l.pad_conv1(stash + Stash::make(*desc).a3 * nb, sp, (int64_t)nb * desc->c2 * 16);
-          HeadArgs ha{sp, packed + g.up2, packed + g.conv2, packed + g.fusedA, w->up2_b, w->conv2_b, w->cls2_b,
+          HeadArgs ha{sp, packed + g.up2, packed + g.conv2, packed + g.cls_is, w->up2_b, w->conv2_b, w->cls2_b,
                       prob_out ? prob_out + b0 * kVox : nullptr, mask + b0 * 1024, counts_out + b0,
                       (float*)(ws + W.off_brow), (float*)(ws + W.off_pl), thh, nb};
           // always one CTA per SM: with fewer (leaf, pass) units than SMs the kernel cuts them along z
           l.head(*desc, ha, l.sms() < kMaxCtas ? l.sms() : kMaxCtas);
         }
-      } else if (is_cfg_A(*desc)) {
-        float* pk = packed + GenericPacked::make(*desc).fusedA;
-        PackParams pp{};
-        pp.job[pp.njobs++] = PackJob{w->conv0_w, pk + FusedA::P_CONV0, PACK_CONVT_FWD, 8, 16, 5};
-        pp.job[pp.njobs++] = PackJob{w->up1_w, pk + FusedA::P_UP1, PACK_CONVT_FWD, 16, 8, 5};
-        pp.job[pp.njobs++] = PackJob{w->conv1_w, pk + FusedA::P_C1, PACK_CONV_FWD, 8, 8, 4};
-        pp.job[pp.njobs++] = PackJob{w->up2_w, pk + FusedA::P_UP2, PACK_CONVT_FWD, 8, 8, 5};
-        pp.job[pp.njobs++] = PackJob{w->conv2_w, pk + FusedA::P_C2, PACK_CONV_FWD, 8, 8, 4};
-        pp.job[pp.njobs++] = PackJob{w->cls2_w, pk + FusedA::P_CLS, PACK_CLS_IS, 1, 8, 3};
-        l.pack(pp);
-        FusedAParams fp{};
-        fp.latent = latent;
-        fp.up0_w = w->up0_w; fp.up0_b = w->up0_b;
-        fp.igdn_beta = w->igdn_beta; fp.igdn_gamma = w->igdn_gamma;
-        fp.conv0_b = w->conv0_b; fp.up1_b = w->up1_b; fp.conv1_b = w->conv1_b;
-        fp.up2_b = w->up2_b; fp.conv2_b = w->conv2_b; fp.cls2_b = w->cls2_b;
-        fp.packed = pk;
-        fp.scratch = (float*)(ws + W.off_scratch);
-        fp.prob_out = prob_out;
-        fp.mask_out = mask;
-        fp.counts_out = counts_out;
-        fp.thh = thh;
-        fp.n_blocks = (int32_t)n_blocks;
-        int grid = l.sms() < kMaxCtas ? l.sms() : kMaxCtas;
-        if (grid > n_blocks) grid = (int)n_blocks;
-        l.fusedA(fp, grid);
       } else {
         pack_all(l, *desc, *w, packed, false, false);
         const int64_t chunk = n_blocks < kGenericDecodeChunk ? n_blocks : kGenericDecodeChunk;
@@ -374,8 +340,7 @@ struct Api {
     l.set_queue(ws + W.off_queue);
     pack_all(l, *desc, *w, packed, true, true);
     forward_layers(l, *desc, *w, packed, latent, (int)n, (float*)(ws + W.off_stash), out, cls1, cls0,
-                   (float*)(ws + W.off_p2), (float*)(ws + W.off_p1), (float*)(ws + W.off_p0), false,
-                   l.train_poly() ? (float*)(ws + W.off_pad) : nullptr);
+                   (float*)(ws + W.off_p2), (float*)(ws + W.off_p1), (float*)(ws + W.off_p0));
     return l.error();
   }
 

@@ -40,42 +40,6 @@ struct SidePool {
 };
 SidePool g_side[kMaxDevices];
 
-
-// Optional programmatic stream serialisation (PDL), NVF_PDL=1: a kernel's CTAs may be scheduled while the
-// previous kernel of the stream is still draining; they block in griddepcontrol.wait (pdl_entry(), first
-// statement of every kernel) until that kernel has completed and flushed, so semantics are those of an
-// ordinary in-order stream.  Measured on B200 (round 1, graph-captured 16-block train step): with every kernel
-// releasing its dependents at entry 0.98 ms vs 0.90 ms without PDL - the early-resident waiting CTAs take the
-// slots the side-stream weight-gradient kernels would otherwise fill; with the heavy kernels releasing them only
-// after their main loop (pdl_entry_heavy / pdl_trigger) 0.899 ms vs 0.891 ms - neutral, the captured graph already
-// hides launch latency - so the default stays OFF (plain launches; the PDL instructions are then no-ops).
-// NVF_ROWS=0 switches the row-register-tile kernels (nvf_rows_*.cuh) off and the smem-tile kernels back on (A/B runs)
-bool rows_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("NVF_ROWS");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
-}
-// NVF_DECODE_HEAD=0 switches the warp-specialised fused decode head off (round-1 phase kernel for 8,16,8,8, layer
-// kernels otherwise) for A/B runs
-bool head_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("NVF_DECODE_HEAD");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
-}
-bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("NVF_PDL");
-    v = (e && e[0] == '1') ? 1 : 0;
-  }
-  return v == 1;
-}
 template <class... KArgs, class... Args>
 void nvf_launch(void (*k)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg{};
@@ -83,11 +47,6 @@ void nvf_launch(void (*k)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStr
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
   cudaLaunchKernelEx(&cfg, k, KArgs(args)...);   // errors are picked up by the caller's cudaGetLastError()
 }
 
@@ -103,26 +62,16 @@ struct DevEnv {
 
 // ------------------------------------------------------------------ kernels
 __global__ void __launch_bounds__(kThreads) k_pack(PackParams p) {
-  pdl_entry();
   pack_thread(p, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x, (int)blockIdx.y);
 }
 
-__global__ void __launch_bounds__(kThreads, 1) k_decode_fused_A(FusedAParams p) {
-  pdl_entry();
-  extern __shared__ __align__(128) float smem[];
-  DevEnv<FusedATS> env;
-  FusedABlock<DevEnv<FusedATS>>::run(env, p, smem, blockIdx.x, gridDim.x);
-}
-
 __global__ void __launch_bounds__(kThreads) k_scan_counts(EmitParams p) {
-  pdl_entry();
   __shared__ int64_t sm[2 * kThreads];
   DevEnv<int> env;
   ScanBlock<DevEnv<int>>::run(env, p, sm);
 }
 
 __global__ void __launch_bounds__(kThreads) k_emit_coords(EmitParams p) {
-  pdl_entry();
   __shared__ int sm[2 * kThreads];
   DevEnv<int> env;
   EmitBlock<DevEnv<int>>::run(env, p, sm, blockIdx.x);
@@ -130,34 +79,29 @@ __global__ void __launch_bounds__(kThreads) k_emit_coords(EmitParams p) {
 
 template <class K>
 __global__ void __launch_bounds__(kThreads) k_generic(typename K::Params p) {
-  pdl_entry();
   K::thread(p, blockIdx.x, threadIdx.x, gridDim.x);
 }
 
 template <int COT, int K>
 __global__ void __launch_bounds__(kThreads) k_wgrad(WgradParams p) {
-  pdl_entry();
   extern __shared__ __align__(128) float smem[];
   DevEnv<int> env;
   WgradBlock<COT, K>::run(env, p, smem, blockIdx.x);
 }
 
 __global__ void __launch_bounds__(kThreads) k_chansum(ChanSumParams p) {
-  pdl_entry();
   __shared__ float sm[kThreads];
   DevEnv<int> env;
   ChanSumBlock::run(env, p, sm, blockIdx.x);
 }
 
 __global__ void __launch_bounds__(kThreads) k_mask(MaskParams p) {
-  pdl_entry();
   __shared__ int sm[kThreads];
   DevEnv<int> env;
   MaskBlock::run(env, p, sm, blockIdx.x);
 }
 
 __global__ void __launch_bounds__(kThreads) k_loss(LossParams p) {
-  pdl_entry();
   __shared__ double sm[kThreads * NVF_LOSS_SUMS];
   DevEnv<int> env;
   LossBlock::run(env, p, sm, blockIdx.x);
@@ -166,7 +110,6 @@ __global__ void __launch_bounds__(kThreads) k_loss(LossParams p) {
 // FFMA throughput probes.  variant 0: scalar FFMA, 8x8 register tile (the shape
 // of the conv inner loops); variant 1: packed fma.rn.f32x2 on the same tile.
 __global__ void __launch_bounds__(kThreads) k_ffma(int variant, long long iters, float* sink) {
-  pdl_entry();
   float w[8], a[8];
   for (int i = 0; i < 8; ++i) {
     w[i] = 1.0f + 1e-6f * (threadIdx.x + i);
@@ -295,24 +238,7 @@ struct DevLauncher {
     nvf_launch(k_pack, dim3(32, p.njobs), dim3(kThreads), (size_t)(0), st, p);   // one grid row per job
     post();
   }
-  void fusedA(const FusedAParams& p, int grid) {
-    static bool attr_set = false;
-    if (!attr_set) {
-      if (!chk(cudaFuncSetAttribute(k_decode_fused_A, cudaFuncAttributeMaxDynamicSharedMemorySize, FusedA::SMEM_BYTES)))
-        return;
-      attr_set = true;
-    }
-    nvf_launch(k_decode_fused_A, dim3(grid), dim3(kThreads), (size_t)(FusedA::SMEM_BYTES), st, p);
-    post();
-  }
-  bool has_head(const NvfDesc& d) { return head_enabled() && head_cfg(d); }
-  // NVF_TRAIN_POLY=1: training forward's up1 / up2 on the polyphase kernel instead of the tile / row kernels.  Off by
-  // default: at 16 blocks it does not pay (up2 45.5 vs 49 us, up1 34.8 vs 25 us, step 0.740 vs 0.732 ms on B200)
-  bool train_poly() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("NVF_TRAIN_POLY"); v = (e && e[0] == '1') ? 1 : 0; }
-    return v == 1;
-  }
+  bool has_head(const NvfDesc& d) { return head_cfg(d); }
   void zero_ints(int32_t* p, int64_t n) { chk(cudaMemsetAsync(p, 0, sizeof(int32_t) * (size_t)n, st)); }
   void pad_conv1(const float* src, float* dst, int64_t planes) {
     int64_t grid = (planes * (fast::kSpPlane / 4) + 255) / 256;
@@ -337,17 +263,10 @@ struct DevLauncher {
     post();
     return true;
   }
-  // up1 of the decode stem (many leaves) and up1 / up2 of the training forward: polyphase kernel on a zero-padded
-  // copy of the input; false = not instantiated for this shape.  Decode uses it for EVERY batch size (a leaf's result
-  // must not depend on it).
+  // up1 of the decode stem: polyphase kernel on a zero-padded copy of the input; false = not instantiated for this
+  // shape.  Decode uses it for EVERY batch size (a leaf's result must not depend on it).
   bool up_poly(const LayerParams& p, float* pad) {
-    if (p.act != ACT_RELU || p.op != OP_CONVT || p.P != 0) return false;
-    if (p.Din == 16) {
-      if (p.CI == 8 && p.CO == 8) return poly_t<8, 8, 16>(p, pad);
-      if (p.CI == 16 && p.CO == 16) return poly_t<16, 16, 16>(p, pad);
-      return false;
-    }
-    if (p.Din != 8) return false;
+    if (p.act != ACT_RELU || p.op != OP_CONVT || p.P != 0 || p.Din != 8) return false;
     // measured on B200, 1247 leaves, vs the tile kernel: 32 -> 16 channels 5.51 -> 3.73 ms, 16 -> 8 channels 1.28 -> 0.98 ms
     if (p.CI == 32 && p.CO == 16) return poly_t<32, 16, 8>(p, pad);
     if (p.CI == 16 && p.CO == 8) return poly_t<16, 8, 8>(p, pad);
@@ -535,17 +454,12 @@ struct DevLauncher {
       return false;
     }
     if (p.op == OP_CONVT && p.P == 0 && p.act == ACT_RELU && !p.add && !p.mask && !p.out2) {
-      if (rows_enabled() && queue_base) {
-        bool done = false;
-        // measured on B200 (16-block step): up2 (8,8,16) 60 -> 54 us; up1 (16,8,8) loses (25 -> 33 us: too little
-        // work per warp item against the per-CTA weight staging), so it stays on the tile kernel
-        if (p.CI == 8 && p.CO == 8 && p.Din == 16) done = convT_fwd_rows<8, 8, 16, 2, 256, 2, false, false>(p);
-        else if (p.CI == 16 && p.CO == 16 && p.Din == 16) done = convT_fwd_rows<16, 16, 16, 2, 256, 1>(p);
-        if (done) return true;
-      }
-      if (p.CI == 8 && p.CO == 8 && p.Din == 16) return convT_fwd<8, 8, 16, 2>(p);
+      // up2 on the queue-fed row kernels (no queue slot: the generic kernel).  Measured on B200 (16-block step): up2
+      // (8,8,16) 60 -> 54 us against the tile kernel; up1 (16,8,8) loses (25 -> 33 us: too little work per warp item
+      // against the per-CTA weight staging), so it stays on the tile kernel
+      if (p.CI == 8 && p.CO == 8 && p.Din == 16) return convT_fwd_rows<8, 8, 16, 2, 256, 2, false, false>(p);
+      if (p.CI == 16 && p.CO == 16 && p.Din == 16) return convT_fwd_rows<16, 16, 16, 2, 256, 1>(p);
       if (p.CI == 16 && p.CO == 8 && p.Din == 8) return convT_fwd<16, 8, 8, 2, 4>(p);
-      if (p.CI == 16 && p.CO == 16 && p.Din == 16) return convT_fwd<16, 16, 16, 1>(p);
       if (p.CI == 32 && p.CO == 16 && p.Din == 8) return convT_fwd<32, 16, 8, 1>(p);
       return false;
     }
@@ -752,12 +666,12 @@ int nvf_last_cuda_error(void) { return g_last_cuda; }
 
 long long nvf_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 
-int nvf_has_fused_decode(const NvfDesc* desc) { return desc && ((head_enabled() && head_cfg(*desc)) || is_cfg_A(*desc)) ? 1 : 0; }
+int nvf_has_fused_decode(const NvfDesc* desc) { return desc && head_cfg(*desc) ? 1 : 0; }
 
 int nvf_workspace_bytes(const NvfDesc* desc, int64_t n_blocks, int mode, size_t* bytes_out) {
   if (!desc || !bytes_out || n_blocks < 0) return NVF_ERR_INVALID_ARG;
   if (!generic_supported(*desc)) return NVF_ERR_UNSUPPORTED;
-  if (mode == NVF_MODE_DECODE) *bytes_out = DecodeWs::make(*desc, n_blocks, head_enabled() && head_cfg(*desc)).total;
+  if (mode == NVF_MODE_DECODE) *bytes_out = DecodeWs::make(*desc, n_blocks, head_cfg(*desc)).total;
   else if (mode == NVF_MODE_TRAIN) *bytes_out = TrainWs::make(*desc, n_blocks).total;
   else return NVF_ERR_INVALID_ARG;
   return NVF_OK;
@@ -1267,7 +1181,7 @@ int train_step_impl(DevLauncher& l, const NvfStepArgs& a, void* workspace, size_
   float* p0 = (float*)(tws + T.off_p0);
   l.set_queue(tws + T.off_queue);   // zero since the caller's one-time fill; every queue-fed kernel rewinds its words
   Api<DevLauncher>::forward_layers(l, d, w, (const float*)(tws + T.off_packed), latent, n, (float*)(tws + T.off_stash), p2, p1, p0,
-                                   nullptr, nullptr, nullptr, false, l.train_poly() ? (float*)(tws + T.off_pad) : nullptr);
+                                   nullptr, nullptr, nullptr);
 
   // ---- loss, metrics, dL/dlogit, total loss and scalar cotangents: one launch
   const bool bwd = wg || demb;

@@ -120,43 +120,10 @@ NVF_HD void p2_load_w8(const float* wp, p2 (&w)[4]) {
   p2_ld2(wp + 4, w[2], w[3]);
 }
 
-// Programmatic dependent launch (only in effect when the launch carries the PDL attribute, NVF_PDL=1).
-//   pdl_entry()       first statement of every kernel: wait until the PREVIOUS kernel of the stream has completed and
-//                     its writes are visible.  Small kernels also release their dependents right away.
-//   pdl_entry_heavy() the long-running kernels wait only; they call pdl_trigger() after their main loop, so the
-//                     next kernel's CTAs are scheduled into the SMs this kernel's tail frees up instead of sitting
-//                     resident (and holding registers / shared memory) for its whole duration.
-#if defined(__CUDA_ARCH__)
-NVF_D void pdl_entry() {
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-}
-NVF_D void pdl_entry_heavy() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-NVF_D void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-#else
-inline void pdl_entry() {}
-inline void pdl_entry_heavy() {}
-inline void pdl_trigger() {}
-#endif
-
 NVF_HD float relu(float v) { return v > 0.f ? v : 0.f; }
 // torch.sigmoid in fp32: 1/(1+exp(-x))
 NVF_HD float sigmoidf(float v) { return 1.f / (1.f + expf(-v)); }
 
-NVF_HD void atomic_or_u32(uint32_t* p, uint32_t v) {
-#if defined(__CUDA_ARCH__)
-  atomicOr(p, v);
-#else
-  *p |= v;
-#endif
-}
-NVF_HD void atomic_add_i32(int* p, int v) {
-#if defined(__CUDA_ARCH__)
-  atomicAdd(p, v);
-#else
-  *p += v;
-#endif
-}
 NVF_HD void atomic_add_f32(float* p, float v) {
 #if defined(__CUDA_ARCH__)
   atomicAdd(p, v);

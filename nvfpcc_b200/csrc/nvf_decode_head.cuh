@@ -497,7 +497,6 @@ __device__ __forceinline__ void head_producer(const HeadParams& p, float* sm, ui
 
 template <int C2, int C3>
 __global__ void __launch_bounds__(kHeadThreads, 1) k_decode_head(HeadParams p) {
-  pdl_entry();
   using G = HeadCfg<C2, C3>;
   extern __shared__ __align__(128) float sm[];
   const int tid = threadIdx.x;
@@ -541,7 +540,6 @@ __global__ void __launch_bounds__(kHeadThreads, 1) k_decode_head(HeadParams p) {
 // from the other pass's conv2 row, then sigmoid / threshold / mask word / point count as in the head kernel.
 template <int C3>
 __global__ void __launch_bounds__(256) k_head_fixup(HeadParams p) {
-  pdl_entry();
   constexpr int RY = 16;
   __shared__ float s_w[C3 * 36];
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
@@ -583,7 +581,6 @@ __global__ void __launch_bounds__(256) k_head_fixup(HeadParams p) {
 // destination per thread): the layout the polyphase transposed-conv tiles read their 6-float windows from
 template <int DIN>
 __global__ void __launch_bounds__(256) k_pad_in(const float* __restrict__ src, float* __restrict__ dst, long long planes) {
-  pdl_entry();
   constexpr int ROWS = DIN + 4, P4 = (DIN + 8) / 4, PL4 = ROWS * P4;
   const long long total = planes * PL4;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -597,8 +594,7 @@ __global__ void __launch_bounds__(256) k_pad_in(const float* __restrict__ src, f
   }
 }
 
-// Stand-alone polyphase k=5 stride-2 transposed conv + ReLU (up1 of the decode stem over many leaves; up1 / up2 of
-// the training forward): the head producer's thread tile (8 x = 4 even + 4 odd outputs, 8 output channels) with one
+// Stand-alone polyphase k=5 stride-2 transposed conv + ReLU (up1 of the decode stem): the head producer's thread tile (8 x = 4 even + 4 odd outputs, 8 output channels) with one
 // WARP ITEM per (leaf, row parity, output slice, channel group, group of RPW rows): up to 32 tiles of equal tap count.
 // Weights stay resident in shared memory when they fit 72 KB - the warps then pull items independently and never
 // meet - else they stream through a two-stage cp.async ring, one input channel at a time, and the four warps of a CTA
@@ -633,7 +629,6 @@ struct PolyParams {
 
 template <int CI, int CO, int DIN>
 __global__ void __launch_bounds__((PolyCfg<CI, CO, DIN>::THREADS), (PolyCfg<CI, CO, DIN>::MINB)) k_convT5_poly(PolyParams p) {
-  pdl_entry();
   using G = PolyCfg<CI, CO, DIN>;
   extern __shared__ __align__(128) float sm[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -725,7 +720,6 @@ __global__ void __launch_bounds__((PolyCfg<CI, CO, DIN>::THREADS), (PolyCfg<CI, 
 
 // conv1 output [n][C][16][16][16] -> zero-padded [n][C][16][20][24] (one float4 of the destination per thread)
 __global__ void __launch_bounds__(256) k_pad_conv1(const float* __restrict__ src, float* __restrict__ dst, long long planes) {
-  pdl_entry();
   const long long total = planes * (kSpPlane / 4);
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const long long pl = i / (kSpPlane / 4);

@@ -162,7 +162,6 @@ __device__ __forceinline__ void conv_s1_chunk(const float* __restrict__ s_in, co
 template <int K, int CI, int C, int DIN, int PAD, int XG, int TY, int NZP, int CIC, int MINB, bool TMA, int COTP = 0>
 __global__ void __launch_bounds__(ConvS1Cfg<K, CI, C, DIN, PAD, XG, TY, NZP, CIC, 0, COTP>::THREADS, MINB)
     k_conv_s1(const __grid_constant__ CUtensorMap tmap, ConvS1Params p) {
-  pdl_entry_heavy();
   constexpr int XSH = TMA ? (4 - PAD % 4) % 4 : 0;
   using G = ConvS1Cfg<K, CI, C, DIN, PAD, XG, TY, NZP, CIC, XSH, COTP>;
   constexpr int COT = G::COT;
@@ -282,7 +281,6 @@ __global__ void __launch_bounds__(ConvS1Cfg<K, CI, C, DIN, PAD, XG, TY, NZP, CIC
     if (active) conv_s1_chunk<G, K, C, CIC, COT, CP, PAIR, XSH>(s_in, s_w, zp, ty, xg, cg, acc2, acc);
   }
   }
-  pdl_trigger();   // main loop done: let the next kernel's CTAs take the SMs this grid's tail frees
   if constexpr (PAIR) {
 #pragma unroll
     for (int a = 0; a < 2; ++a)
@@ -374,7 +372,6 @@ struct WgradS1Cfg {
 
 template <int C, int DG, int TYG, int MINB>
 __global__ void __launch_bounds__(256, MINB) k_wgrad4_s1(WgradS1Params p) {
-  pdl_entry_heavy();
   using G = WgradS1Cfg<C, DG, TYG>;
   extern __shared__ __align__(128) float smem[];
   float* s_a = smem;
@@ -473,7 +470,6 @@ __global__ void __launch_bounds__(256, MINB) k_wgrad4_s1(WgradS1Params p) {
       }
     }
   }
-  pdl_trigger();
   // ---- CTA result: sum the position sets, write one partial in PyTorch layout (co,ci,kz,ky,kx)
   float acc[8][2][4];
 #pragma unroll
@@ -537,7 +533,6 @@ struct ReduceParams {
 };
 // grid.y = job; 8 lanes along the partial index x 32 outputs per CTA
 __global__ void __launch_bounds__(256) k_reduce_partials(ReduceParams p) {
-  pdl_entry();
   __shared__ float sm[8][33];
   const ReduceJob& J = p.job[blockIdx.y];
   const int n = J.n_w + J.n_b;

@@ -49,7 +49,6 @@ struct ConvTFwdCfg {
 
 template <int CI, int CO, int DIN, int MINB, int KS = 1>
 __global__ void __launch_bounds__(ConvTFwdCfg<CI, CO, DIN, KS>::THREADS, MINB) k_convT5_fwd(ConvTFwdParams p) {
-  pdl_entry_heavy();
   using G = ConvTFwdCfg<CI, CO, DIN, KS>;
   extern __shared__ __align__(128) float smem[];
   float* s_in = smem;
@@ -159,7 +158,6 @@ __global__ void __launch_bounds__(ConvTFwdCfg<CI, CO, DIN, KS>::THREADS, MINB) k
       }
     }
   }
-  pdl_trigger();
   float acc[2][4][8];
 #pragma unroll
   for (int a = 0; a < 2; ++a)
@@ -252,7 +250,6 @@ struct ConvTDgradCfg {
 
 template <int CG, int CX, int DIN, int TY, int CGC, int MINB>
 __global__ void __launch_bounds__(ConvTDgradCfg<CG, CX, DIN, TY, CGC>::THREADS, MINB) k_convT5_dgrad(ConvTDgradParams p) {
-  pdl_entry_heavy();
   using G = ConvTDgradCfg<CG, CX, DIN, TY, CGC>;
   extern __shared__ __align__(128) float smem[];
   const int tid = threadIdx.x;
@@ -352,7 +349,6 @@ __global__ void __launch_bounds__(ConvTDgradCfg<CG, CX, DIN, TY, CGC>::THREADS, 
     tma::cp_async_wait_all();
     __syncthreads();   // next chunk has landed; everyone is done with this one
   }
-  pdl_trigger();
   float acc[2][8][4];
 #pragma unroll
   for (int a = 0; a < 2; ++a)
@@ -437,7 +433,6 @@ struct ConvTWgradCfg {
 
 template <int CI, int CO, int DIN, int TYB, int CIB, int MINB>
 __global__ void __launch_bounds__(224, MINB) k_convT5_wgrad(ConvTWgradParams p) {
-  pdl_entry_heavy();
   using G = ConvTWgradCfg<CI, CO, DIN, TYB, CIB>;
   extern __shared__ __align__(128) float smem[];
   float* s_g = smem;
@@ -519,7 +514,6 @@ __global__ void __launch_bounds__(224, MINB) k_convT5_wgrad(ConvTWgradParams p) 
       }
     }
   }
-  pdl_trigger();
   if (!active) return;
   // partial in the layout [ci_local][co_local][kz][ky][kx]
   float* out = p.partial + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * G::OUT_FLOATS;
@@ -540,7 +534,6 @@ struct ChanSumFastParams {
   int32_t n, C, D, P, ZCH;  // ZCH chunks along z
 };
 __global__ void __launch_bounds__(256) k_chansum_fast(ChanSumFastParams p) {
-  pdl_entry();
   __shared__ float sm[256];
   const int c = blockIdx.x % p.C;
   const int zc = (blockIdx.x / p.C) % p.ZCH;

@@ -130,7 +130,6 @@ __device__ __forceinline__ void latent_load_params(const LatentKParams& p, float
 
 template <int CH>
 __global__ void __launch_bounds__(kLatentThreads) k_latent_fwd(LatentKParams p) {
-  pdl_entry();
   __shared__ double sm[kLatentThreads / 32];
   float W[CH][CH], bias[CH], beta[CH], gamma[CH][CH];
   latent_load_params<CH>(p, W, bias, beta, gamma);
@@ -159,7 +158,6 @@ __global__ void __launch_bounds__(kLatentThreads) k_latent_fwd(LatentKParams p) 
 
 template <int CH>
 __global__ void __launch_bounds__(kLatentThreads) k_latent_bwd(LatentKParams p) {
-  pdl_entry();
   constexpr int NP = LatentCfg<CH>::NP_BWD;
   float W[CH][CH], bias[CH], beta[CH], gamma[CH][CH];
   latent_load_params<CH>(p, W, bias, beta, gamma);
@@ -289,7 +287,6 @@ struct RdTotalParams {
 
 template <bool BWD>
 __global__ void k_rd_total(RdTotalParams p) {
-  pdl_entry();
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   if (!BWD) {
     const float bce = (float)p.sums[0], ms0 = (float)p.sums[1], ms1 = (float)p.sums[2];
@@ -355,7 +352,6 @@ struct AdamParams {
 };
 
 __global__ void __launch_bounds__(256) k_adam(AdamParams p) {
-  pdl_entry();
   float step_size, bc2s;
   adam_bias_corrections(p.step, p.lr, p.beta1, p.beta2, step_size, bc2s);
   for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < p.n; i += (int64_t)gridDim.x * 256) {
@@ -367,7 +363,6 @@ __global__ void __launch_bounds__(256) k_adam(AdamParams p) {
 }
 // the counter is advanced by a separate one-thread launch so every CTA of k_adam sees the same t
 __global__ void k_adam_tick(float* step) {
-  pdl_entry();
   step[0] += 1.f;
 }
 

@@ -43,7 +43,6 @@ struct ClsWgradCfg {
 
 template <int C, int D, int TYB, int ZSEG>
 __global__ void __launch_bounds__(256) k_cls_wgrad(ClsWgradParams p) {
-  pdl_entry();
   using G = ClsWgradCfg<C, D, TYB, ZSEG>;
   extern __shared__ __align__(128) float smem[];
   float* s_a = smem;
@@ -165,7 +164,6 @@ struct IgdnParamParams {
   int32_t n, C;
 };
 __global__ void __launch_bounds__(256) k_igdn_param(IgdnParamParams p) {
-  pdl_entry();
   extern __shared__ __align__(128) float smem[];
   const int C = p.C;
   float* sx2 = smem;             // [C][64]  x^2

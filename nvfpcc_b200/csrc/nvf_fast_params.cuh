@@ -96,7 +96,6 @@ __device__ __forceinline__ float cta_sum_256(float v, float* sm) {
 
 template <bool BWD>
 __global__ void __launch_bounds__(256) k_param_prep(ParamPrepParams p) {
-  pdl_entry();
   __shared__ float sm[8];
   const int tid = threadIdx.x;
   if ((int)blockIdx.x == p.total_chunks) {
@@ -194,7 +193,6 @@ __global__ void __launch_bounds__(256) k_param_prep(ParamPrepParams p) {
 
 template <bool BWD>
 __global__ void __launch_bounds__(32) k_param_final(ParamPrepParams p) {
-  pdl_entry();
   param_finalise<BWD>(p, (int)threadIdx.x);
 }
 

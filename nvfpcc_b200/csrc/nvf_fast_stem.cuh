@@ -47,7 +47,6 @@ __device__ __forceinline__ int stem_tap_lo(int o) { return o & 1; }
 constexpr int kStemFwdThreads = 512;
 template <bool PERSIST>
 __global__ void __launch_bounds__(kStemFwdThreads) k_stem_fwd(StemFwdParams p) {
-  pdl_entry();
   extern __shared__ __align__(128) float smem[];
   const int CH = p.CH, C0 = p.C0, C1 = p.C1;
   float* s_lat = smem;                 // [CH][8]
@@ -176,7 +175,6 @@ __host__ __device__ inline int stem_partial_floats(int CH, int C0, int C1) {
 //   conv0 dgrad gy[b][ci][64] -> p.gy (global).
 constexpr int kStemBwdAThreads = 512;   // these kernels are latency-bound chains: more threads = shorter chains
 __global__ void __launch_bounds__(kStemBwdAThreads) k_stem_bwd_a(StemBwdParams p, float* gy_out) {
-  pdl_entry();
   extern __shared__ __align__(128) float smem[];
   const int CH = p.CH, C0 = p.C0, C1 = p.C1;
   float* s_g1 = smem;                   // [C1][512]
@@ -261,7 +259,6 @@ __global__ void __launch_bounds__(kStemBwdAThreads) k_stem_bwd_a(StemBwdParams p
 // Kernel B, grid = n: IGDN backward (dx, dbeta, dgamma), up0 wgrad / bias, d_latent.
 constexpr int kStemBwdBThreads = 1024;
 __global__ void __launch_bounds__(kStemBwdBThreads) k_stem_bwd_b(StemBwdParams p, const float* gy_in) {
-  pdl_entry();
   extern __shared__ __align__(128) float smem[];
   const int CH = p.CH, C0 = p.C0, C1 = p.C1;
   float* s_x0 = smem;                   // [C0][64]

@@ -76,7 +76,6 @@ __device__ __forceinline__ int cell_lookup(const CellTable& T, int c0, int c1, i
 
 // Pass 1a: every point claims the hash slot of its cell; the first claimant numbers the cell.
 __global__ void __launch_bounds__(256) k_cells_insert(const int32_t* __restrict__ pts, int64_t n, CellTable T) {
-  pdl_entry();
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     unsigned long long key;
     if (!cell_key(pts[3 * i] >> 5, pts[3 * i + 1] >> 5, pts[3 * i + 2] >> 5, key)) {
@@ -104,7 +103,6 @@ __global__ void __launch_bounds__(256) k_cells_insert(const int32_t* __restrict_
 
 // Pass 1b: set the point's bit in its cell.
 __global__ void __launch_bounds__(256) k_points_scatter(const int32_t* __restrict__ pts, int64_t n, CellTable T) {
-  pdl_entry();
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const int a0 = pts[3 * i], a1 = pts[3 * i + 1], a2 = pts[3 * i + 2];
     const int id = cell_lookup(T, a0 >> 5, a1 >> 5, a2 >> 5);
@@ -261,7 +259,6 @@ __device__ __forceinline__ int isqrt_floor(uint32_t v) {
 }
 
 __global__ void __launch_bounds__(kThreads, 2) k_edt_blocks(EdtParams p) {
-  pdl_entry();
   extern __shared__ __align__(16) unsigned char smem_raw[];
   EdtSmem& S = *reinterpret_cast<EdtSmem*>(smem_raw);
   const int tid = threadIdx.x;

@@ -497,7 +497,7 @@ struct Stash {
 struct GenericPacked {
   int64_t conv0, up1, conv1, up2, conv2, cls2, cls1, cls0;              // forward packs (up0 uses PACK_CONVT_FWD too)
   int64_t up0, d_up0, d_conv0, d_up1, d_conv1, d_up2, d_conv2, d_cls2, d_cls1, d_cls0;
-  int64_t fusedA;  // FusedA::PACKED_FLOATS region for the fused decode kernel
+  int64_t cls_is;  // PACK_CLS_IS copy of cls2 for the fused decode head
   int64_t total;
   static GenericPacked make(const NvfDesc& d) {
     GenericPacked g{};
@@ -521,7 +521,7 @@ struct GenericPacked {
     g.d_cls2 = take((int64_t)d.c3 * 27);
     g.d_cls1 = take((int64_t)d.c2 * 27);
     g.d_cls0 = take((int64_t)d.c1 * 27);
-    g.fusedA = take(65536);
+    g.cls_is = take((int64_t)d.c3 * 36);
     g.total = o;
     return g;
   }

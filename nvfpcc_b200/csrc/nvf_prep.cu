@@ -57,7 +57,6 @@ __global__ void __launch_bounds__(256) k_gather_batch(const float* __restrict__ 
                                                       int64_t n_rows, int emb_floats, float* __restrict__ emb_out,
                                                       float4* __restrict__ gt_out, float4* __restrict__ dist_out,
                                                       int32_t* __restrict__ status) {
-  pdl_entry();
   const int b = blockIdx.x, part = blockIdx.y;
   int64_t row = idx[b];
   if (row < 0 || row >= n_rows) {

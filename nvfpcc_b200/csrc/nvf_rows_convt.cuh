@@ -74,7 +74,6 @@ __device__ __forceinline__ void row_step(p2 (&acc)[DOUT], const float4 (&r)[DIN 
 // rows of one block and class and share their input rows in L1 (items of one class cost the same)
 template <int CI, int CO, int DIN, int KS, int THREADS, int MINB, bool PIPE = false, bool CHUNK = true>
 __global__ void __launch_bounds__(THREADS, MINB) k_convT5_fwd_rows(RowTFwdParams p) {
-  pdl_entry_heavy();
   using G = RowTFwdCfg<CI, CO, DIN, KS>;
   extern __shared__ __align__(128) float s_w[];
   const int tid = threadIdx.x, lane = tid & 31;
@@ -216,7 +215,6 @@ __global__ void __launch_bounds__(THREADS, MINB) k_convT5_fwd_rows(RowTFwdParams
       }
     }
   }
-  pdl_trigger();
   // ---- retire: the last warp / CTA of the grid to run dry rewinds the queue for the next launch
   if (CHUNK ? tid == 0 : lane == 0) {
     const unsigned d = atomicAdd(p.queue + 1, 1u);

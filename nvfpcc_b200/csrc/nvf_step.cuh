@@ -40,7 +40,6 @@ struct LossStepParams {
 };
 
 __global__ void __launch_bounds__(256) k_loss_step(LossStepParams p) {
-  pdl_entry();
   __shared__ double sm[8][NVF_LOSS_SUMS];
   const int tid = threadIdx.x;
   const int b = blockIdx.x / kLossChunks, chunk = blockIdx.x % kLossChunks;
@@ -168,7 +167,6 @@ __global__ void __launch_bounds__(256) k_loss_step(LossStepParams p) {
 
 // advances the device-resident step counter of the in-kernel noise generators (one thread, end of the step)
 __global__ void k_rng_tick(unsigned long long* ctr) {
-  pdl_entry();
   ctr[0] += 1ull;
 }
 

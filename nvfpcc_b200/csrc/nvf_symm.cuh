@@ -55,7 +55,6 @@ __device__ __forceinline__ float4 ld_volatile_f4(const float4* p) {
 
 // grid <= 64 CTAs (all resident: the last CTA to finish its copy publishes for the whole grid)
 __global__ void __launch_bounds__(256) k_allreduce_adam(ArAdamParams p) {
-  pdl_entry();
   const int tid = threadIdx.x;
   const unsigned int seq = *(volatile unsigned int*)p.ctl + 1u;
   const size_t boff = (size_t)(seq & 1u) * p.n4;

@@ -84,36 +84,6 @@ NVF_HD void corr_s1_tile(const View& in, int CI, int P, const float* Wp, int CO,
   }
 }
 
-// Valid (no padding) k=4 correlation with aligned 128-bit activation loads:
-// requires ox0 % 4 == 0, ys % 4 == 0, base 16-byte aligned and ox0+7 < row pitch.
-template <int COT>
-NVF_HD void conv4_valid_tile(const View& in, int CI, const float* Wp, int CO, int co0, int oz, int oy, int ox0,
-                             float (&acc)[COT][4]) {
-  NVF_NOUNROLL
-  for (int ci = 0; ci < CI; ++ci) {
-    NVF_NOUNROLL
-    for (int kz = 0; kz < 4; ++kz) {
-      NVF_UNROLL
-      for (int ky = 0; ky < 4; ++ky) {
-        const float* row = in.base + ci * in.cs + (oz + kz) * in.zs + (oy + ky) * in.ys + ox0;
-        const f4 lo = ld4(row), hi = ld4(row + 4);
-        const float a[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
-        const float* wrow = Wp + (((ci * 4 + kz) * 4 + ky) * 4) * CO + co0;
-        NVF_UNROLL
-        for (int kx = 0; kx < 4; ++kx) {
-          float w[COT];
-          load_w<COT>(wrow + kx * CO, w);
-          NVF_UNROLL
-          for (int c = 0; c < COT; ++c) {
-            NVF_UNROLL
-            for (int j = 0; j < 4; ++j) acc[c][j] = fmaf(w[c], a[j + kx], acc[c][j]);
-          }
-        }
-      }
-    }
-  }
-}
-
 // Transposed conv k5 s2, padding P in {0,2}: 4 consecutive outputs ox0..ox0+3
 // (ox0 % 4 == 0, so outputs 0,2 use even kx and 1,3 odd kx).
 template <int COT>

@@ -23,5 +23,5 @@ torch.cuda.synchronize()
 c = r["coords"].cpu().long()
 w = torch.arange(1, c.shape[0] + 1, dtype=torch.int64) % 1000003
 chk = int(((c * torch.tensor([1, 1 << 11, 1 << 22])).sum(1) * w).sum() % (1 << 61))
-print("HEAD=%s %s res %d: %d leaves, %.3f ms per decode, %d points, checksum %d" % (
-    os.environ.get("NVF_DECODE_HEAD", "1"), chanstr, res, dw.n_all, e0.elapsed_time(e1) / reps, c.shape[0], chk))
+print("%s res %d: %d leaves, %.3f ms per decode, %d points, checksum %d" % (
+    chanstr, res, dw.n_all, e0.elapsed_time(e1) / reps, c.shape[0], chk))

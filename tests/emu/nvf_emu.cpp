@@ -1,11 +1,14 @@
 // TEST-ONLY CPU emulator of the NVF kernels.
 //
-// Compiles the SAME kernel bodies and host orchestration as the CUDA library
-// (nvfpcc_b200/csrc/*.h) with g++, executing every CTA's threads sequentially
-// phase by phase (a phase boundary is a __syncthreads()).  It lets the
-// `-m "not gpu"` tests check index arithmetic, workspace layouts and sequencing
-// against the oracle before GPU time is spent.  It is NOT part of the product:
-// nvfpcc_b200 never loads it and there is no CPU fallback in the package.
+// Compiles the SAME generic kernel bodies (nvf_layers.h, nvf_emit.h) and host
+// orchestration (nvf_api_impl.h) as the CUDA library with g++, executing every
+// CTA's threads sequentially phase by phase (a phase boundary is a
+// __syncthreads()).  The fused decode head and the shared-memory tiled kernels
+// are CUDA-only, so here decode and training run layer-wise for every
+// configuration.  It lets the `-m "not gpu"` tests check index arithmetic,
+// workspace layouts and sequencing against the oracle before GPU time is spent.
+// It is NOT part of the product: nvfpcc_b200 never loads it and there is no CPU
+// fallback in the package.
 #include <stdlib.h>
 #include <string.h>
 #include <vector>
@@ -35,14 +38,6 @@ struct EmuLauncher {
     const int g = 4 * kThreads;
     for (int t = 0; t < g; ++t) pack_thread(p, t, g);
   }
-  void fusedA(const FusedAParams& p, int grid) {
-    std::vector<float> sm(FusedA::SMEM_FLOATS);
-    for (int cta = 0; cta < grid; ++cta) {
-      for (auto& v : sm) v = 1e30f;  // poison: uninitialised smem must never be consumed
-      EmuEnv<FusedATS> env;
-      FusedABlock<EmuEnv<FusedATS>>::run(env, p, sm.data(), cta, grid);
-    }
-  }
   void scan(const EmitParams& p) {
     std::vector<int64_t> sm(2 * kThreads);
     EmuEnv<int> env;
@@ -63,12 +58,11 @@ struct EmuLauncher {
                      float*, float*, float*, float*, float*) { return false; }
   bool fast_stem_bwd(const NvfDesc&, const NvfWeights&, const float*, int, const float*, const float*, const float*,
                      float*, const NvfWeightGrads*, float*) { return false; }
-  // the warp-specialised fused decode head is CUDA-only: the emulator runs the round-1 phase kernel / layer kernels
+  // the warp-specialised fused decode head is CUDA-only: the emulator decodes with the layer kernels
   bool has_head(const NvfDesc&) { return false; }
   void zero_ints(int32_t*, int64_t) {}
   void pad_conv1(const float*, float*, int64_t) {}
   bool up_poly(const LayerParams&, float*) { return false; }
-  bool train_poly() { return false; }
   void head(const NvfDesc&, const HeadArgs&, int) {}
   void side_begin() {}
   void side_end() {}
@@ -128,7 +122,7 @@ int nvf_abi_version(void) { return NVF_ABI_VERSION; }
 const char* nvf_strerror(int code) { return code == NVF_OK ? "ok" : "error (emulator)"; }
 int nvf_last_cuda_error(void) { return 0; }
 long long nvf_launch_count(void) { return 0; }
-int nvf_has_fused_decode(const NvfDesc* desc) { return desc && is_cfg_A(*desc) ? 1 : 0; }
+int nvf_has_fused_decode(const NvfDesc*) { return 0; }
 
 int nvf_workspace_bytes(const NvfDesc* desc, int64_t n_blocks, int mode, size_t* bytes_out) {
   if (!desc || !bytes_out || n_blocks < 0) return NVF_ERR_INVALID_ARG;

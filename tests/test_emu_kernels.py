@@ -1,6 +1,8 @@
-"""Kernel-logic tests on the CPU emulator (tests/emu): the same kernel bodies and
-host orchestration as the CUDA library, executed sequentially, checked against
-the oracle.  The `-m gpu` tests repeat these checks on the real device."""
+"""Kernel-logic tests on the CPU emulator (tests/emu): the same generic layer kernels,
+point emission and host orchestration as the CUDA library, executed sequentially,
+checked against the oracle.  Decode runs layer-wise here for every configuration
+(the fused decode head is CUDA-only).  The `-m gpu` tests repeat these checks on
+the real device."""
 import numpy as np
 import pytest
 import torch
@@ -16,7 +18,7 @@ def emu():
     return emu_backend.binding()
 
 
-def test_decode_fused_A_matches_oracle_and_golden(emu, golden_A):
+def test_decode_layerwise_A_matches_oracle_and_golden(emu, golden_A):
     fx = fixture_inputs("A")
     lat = torch.cat([fx["latents"], fx["latents"].flip(0) * 0.5 + 1, fx["latents"][:1] * -1.0], 0).round()
     check_decode_against_oracle(emu, fx, lat, thh=0.5, golden=golden_A, dev="cpu")
