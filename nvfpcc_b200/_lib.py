@@ -13,7 +13,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import Dict, Optional, Sequence
+from typing import Callable, Dict, Optional, Sequence
 
 import torch
 
@@ -39,7 +39,11 @@ EXPORTS = (
 LATENT_FIELDS = ("kernel", "kernel_init", "b", "b_init", "gdn_beta", "gdn_gamma", "sigma", "mu")   # NvfLatentParams
 LATENT_GRAD_FIELDS = ("kernel", "b", "gdn_beta", "gdn_gamma", "sigma", "mu")                         # NvfLatentGrads
 NVF_LATENT_WS_BYTES = 128 * 1024
-CONV_LAYERS = ("up0", "conv0", "up1", "conv1", "up2", "conv2", "cls2", "cls1", "cls0")   # NvfParamSet order
+# The decoder's nine convolutions in NvfParamSet order: ABI key -> CompDecoder attribute.  The first NVF_NUM_QUANT
+# are the quantised ones.
+CONV_MODULES = {"up0": "up0", "conv0": "conv0", "up1": "up1", "conv1": "conv1", "up2": "up2", "conv2": "conv2",
+                "cls2": "conv2_cls", "cls1": "conv1_cls", "cls0": "conv0_cls"}
+CONV_LAYERS = tuple(CONV_MODULES)
 NVF_NUM_CONV, NVF_NUM_QUANT, NVF_PARAM_WS_BYTES = 9, 7, 64 * 1024
 
 
@@ -53,17 +57,6 @@ class NvfWeights(C.Structure):
 
 class NvfWeightGrads(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in WEIGHT_FIELDS]
-
-
-def weight_shapes(ch: int, channels: Sequence[int]) -> Dict[str, tuple]:
-    c0, c1, c2, c3 = (int(c) for c in channels)
-    return {
-        "up0_w": (ch, c0, 5, 5, 5), "up0_b": (c0,), "igdn_beta": (c0,), "igdn_gamma": (c0, c0),
-        "conv0_w": (c0, c1, 5, 5, 5), "conv0_b": (c1,), "up1_w": (c1, c2, 5, 5, 5), "up1_b": (c2,),
-        "conv1_w": (c2, c2, 4, 4, 4), "conv1_b": (c2,), "up2_w": (c2, c3, 5, 5, 5), "up2_b": (c3,),
-        "conv2_w": (c3, c3, 4, 4, 4), "conv2_b": (c3,), "cls2_w": (1, c3, 3, 3, 3), "cls2_b": (1,),
-        "cls1_w": (1, c2, 3, 3, 3), "cls1_b": (1,), "cls0_w": (1, c1, 3, 3, 3), "cls0_b": (1,),
-    }
 
 
 class NvfParamSet(C.Structure):
@@ -105,6 +98,17 @@ class NvfError(RuntimeError):
 
 def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def param_set(raw: Dict[str, torch.Tensor], ptr: Callable[[torch.Tensor], int]) -> NvfParamSet:
+    """NvfParamSet over the raw tensors of ops.RAW_FIELDS; ptr(tensor) -> the device address to pass."""
+    ps = NvfParamSet()
+    for i, key in enumerate(CONV_LAYERS):
+        for field in ("kernel", "kernel_init", "b", "b_init"):
+            getattr(ps, field)[i] = ptr(raw["%s_%s" % (key, field)])
+    for field in ("igdn_beta", "igdn_gamma", "lik_sigma", "lik_mu"):
+        setattr(ps, field, ptr(raw[field]))
+    return ps
 
 
 class Binding:
@@ -313,19 +317,12 @@ class Binding:
     # ---- fused parameter-side transforms --------------------------------------------------------
     @staticmethod
     def _param_set(raw: Dict[str, torch.Tensor]):
-        """raw: {layer}_{kernel,kernel_init,b,b_init} for layer in CONV_LAYERS + igdn_beta/igdn_gamma/lik_sigma/lik_mu."""
-        ps = NvfParamSet()
         keep = []
-        for i, name in enumerate(CONV_LAYERS):
-            for field in ("kernel", "kernel_init", "b", "b_init"):
-                t = raw["%s_%s" % (name, field)].detach().contiguous()
-                keep.append(t)
-                getattr(ps, field)[i] = t.data_ptr()
-        for field in ("igdn_beta", "igdn_gamma", "lik_sigma", "lik_mu"):
-            t = raw[field].detach().contiguous()
-            keep.append(t)
-            setattr(ps, field, t.data_ptr())
-        return ps, keep
+
+        def ptr(t):
+            keep.append(t.detach().contiguous())
+            return keep[-1].data_ptr()
+        return param_set(raw, ptr), keep
 
     def param_prep(self, desc: NvfDesc, raw: Dict[str, torch.Tensor], q: int, noise: Optional[torch.Tensor],
                    beta_bound: float, gamma_bound: float, pedestal: float):

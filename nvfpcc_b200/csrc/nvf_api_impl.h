@@ -42,9 +42,8 @@ constexpr int kMaxPartialCtas = 304;          // persistent CTAs of a split-K we
 // writes <= kMaxPartialCtas partial copies of its layer's gradient; per-block partials of the
 // stem / bias sums need n-proportional room.
 inline size_t partial_floats(const NvfDesc& d, int64_t n) {
-  const size_t params = (size_t)d.ch * d.c0 * 125 + (size_t)d.c0 * d.c1 * 125 + (size_t)d.c1 * d.c2 * 125 +
-                        (size_t)d.c2 * d.c3 * 125 + (size_t)d.c2 * d.c2 * 64 + (size_t)d.c3 * d.c3 * 64 +
-                        27 * (size_t)(d.c1 + d.c2 + d.c3) + 2 * (size_t)(d.c0 + d.c1 + d.c2 + d.c3) + 64 * 24;
+  size_t params = 2 * (size_t)(d.c0 + d.c1 + d.c2 + d.c3) + 64 * 24;
+  for (int l = 0; l < NVF_NUM_CONV; ++l) params += (size_t)conv_geom(d, l).n();
   const size_t stem = (size_t)d.c0 * d.c1 * 125 + d.c1 + (size_t)d.c0 * d.c0 + d.c0 + (size_t)d.ch * d.c0 * 125 + d.c0;
   return (size_t)kMaxPartialCtas * params +
          (size_t)n * (stem + (size_t)d.c0 * d.c0 + 8 * (size_t)(d.c0 + d.c1 + d.c2 + d.c3) + 64 * 16);
@@ -152,32 +151,15 @@ struct Api {
   static int pack_all(L& l, const NvfDesc& d, const NvfWeights& w, float* packed, bool fwd_aux, bool dgrad) {
     const GenericPacked g = GenericPacked::make(d);
     PackParams pp{};
-    auto job = [&](const float* src, int64_t off, int mode, int A, int B, int K) {
+    auto job = [&](int i, int64_t off, int mode) {
+      const ConvGeom c = conv_geom(d, i);
       if (pp.njobs == kMaxPackJobs) { l.pack(pp); pp.njobs = 0; }
-      pp.job[pp.njobs++] = PackJob{src, packed + off, mode, A, B, K};
+      pp.job[pp.njobs++] = PackJob{slots(w)[c.slot], packed + off, mode, c.A, c.B, c.K};
     };
-    job(w.up0_w, g.up0, PACK_CONVT_FWD, d.ch, d.c0, 5);
-    job(w.conv0_w, g.conv0, PACK_CONVT_FWD, d.c0, d.c1, 5);
-    job(w.up1_w, g.up1, PACK_CONVT_FWD, d.c1, d.c2, 5);
-    job(w.conv1_w, g.conv1, PACK_CONV_FWD, d.c2, d.c2, 4);
-    job(w.up2_w, g.up2, PACK_CONVT_FWD, d.c2, d.c3, 5);
-    job(w.conv2_w, g.conv2, PACK_CONV_FWD, d.c3, d.c3, 4);
-    job(w.cls2_w, g.cls2, PACK_CONV_FWD, 1, d.c3, 3);
-    if (fwd_aux) {
-      job(w.cls1_w, g.cls1, PACK_CONV_FWD, 1, d.c2, 3);
-      job(w.cls0_w, g.cls0, PACK_CONV_FWD, 1, d.c1, 3);
-    }
-    if (dgrad) {
-      job(w.up0_w, g.d_up0, PACK_CONVT_DGRAD, d.ch, d.c0, 5);
-      job(w.conv0_w, g.d_conv0, PACK_CONVT_DGRAD, d.c0, d.c1, 5);
-      job(w.up1_w, g.d_up1, PACK_CONVT_DGRAD, d.c1, d.c2, 5);
-      job(w.conv1_w, g.d_conv1, PACK_CONV_DGRAD, d.c2, d.c2, 4);
-      job(w.up2_w, g.d_up2, PACK_CONVT_DGRAD, d.c2, d.c3, 5);
-      job(w.conv2_w, g.d_conv2, PACK_CONV_DGRAD, d.c3, d.c3, 4);
-      job(w.cls2_w, g.d_cls2, PACK_CONV_DGRAD, 1, d.c3, 3);
-      job(w.cls1_w, g.d_cls1, PACK_CONV_DGRAD, 1, d.c2, 3);
-      job(w.cls0_w, g.d_cls0, PACK_CONV_DGRAD, 1, d.c1, 3);
-    }
+    for (int i = 0; i < (fwd_aux ? NVF_NUM_CONV : L_CLS1); ++i)
+      job(i, g.fwd[i], conv_geom(d, i).convT ? PACK_CONVT_FWD : PACK_CONV_FWD);
+    if (dgrad)
+      for (int i = 0; i < NVF_NUM_CONV; ++i) job(i, g.dg[i], conv_geom(d, i).convT ? PACK_CONVT_DGRAD : PACK_CONV_DGRAD);
     if (pp.njobs) l.pack(pp);
     return NVF_OK;
   }
@@ -196,30 +178,31 @@ struct Api {
     float* a5 = stash + s.a5 * n;
     LayerParams p{};
     p.n = n;
-    if (!l.fast_stem_fwd(d, w, packed + g.up0, packed + g.conv0, packed + g.cls0, latent, n, x0, a0, a1, cls0, p0)) {
+    if (!l.fast_stem_fwd(d, w, packed + g.fwd[L_UP0], packed + g.fwd[L_CONV0], packed + g.fwd[L_CLS0], latent, n, x0,
+                         a0, a1, cls0, p0)) {
       // up0: convT k5 s2 p2 op1 (utils/network.py:4671-4680)
-      p = LayerParams{latent, x0, packed + g.up0, w.up0_b, nullptr, nullptr, n, d.ch, d.c0, 2, 2, 4, 4, 2, ACT_NONE, OP_CONVT};
+      p = LayerParams{latent, x0, packed + g.fwd[L_UP0], w.up0_b, nullptr, nullptr, n, d.ch, d.c0, 2, 2, 4, 4, 2, ACT_NONE, OP_CONVT};
       layer(l, p);
       IgdnParams ip{x0, a0, nullptr, w.igdn_beta, w.igdn_gamma, nullptr, nullptr, n, d.c0};
       l.template generic<IgdnFwdKernel>(ip, (int)((int64_t)n * d.c0 * 64 + kThreads - 1) / kThreads);
       // conv0: convT k5 s2 p2 op1 + ReLU (:4682-4691, :4760)
-      p = LayerParams{a0, a1, packed + g.conv0, w.conv0_b, nullptr, nullptr, n, d.c0, d.c1, 4, 4, 8, 8, 2, ACT_RELU, OP_CONVT};
+      p = LayerParams{a0, a1, packed + g.fwd[L_CONV0], w.conv0_b, nullptr, nullptr, n, d.c0, d.c1, 4, 4, 8, 8, 2, ACT_RELU, OP_CONVT};
       layer(l, p);
       if (cls0) {  // conv0_cls + sigmoid (:4743-4751, :4761)
-        p = LayerParams{a1, cls0, packed + g.cls0, w.cls0_b, nullptr, nullptr, n, d.c1, 1, 8, 8, 8, 8, 1, ACT_SIGMOID, OP_CORR3};
+        p = LayerParams{a1, cls0, packed + g.fwd[L_CLS0], w.cls0_b, nullptr, nullptr, n, d.c1, 1, 8, 8, 8, 8, 1, ACT_SIGMOID, OP_CORR3};
         p.out2 = p0;
         layer(l, p);
       }
     }
     // up1: convT k5 s2 p0 + ReLU (:4693-4700, :4762)
-    p = LayerParams{a1, a2, packed + g.up1, w.up1_b, nullptr, nullptr, n, d.c1, d.c2, 8, 8, 19, 20, 0, ACT_RELU, OP_CONVT};
+    p = LayerParams{a1, a2, packed + g.fwd[L_UP1], w.up1_b, nullptr, nullptr, n, d.c1, d.c2, 8, 8, 19, 20, 0, ACT_RELU, OP_CONVT};
     // fused-head decode (pad_scratch): polyphase kernel on a zero-padded copy of conv0's output; else the tile kernels
     if (!(pad_scratch && l.up_poly(p, pad_scratch))) layer(l, p);
     // conv1: conv k4 + ReLU (:4702-4710, :4763)
-    p = LayerParams{a2, a3, packed + g.conv1, w.conv1_b, nullptr, nullptr, n, d.c2, d.c2, 19, 20, 16, 16, 0, ACT_RELU, OP_CORR4};
+    p = LayerParams{a2, a3, packed + g.fwd[L_CONV1], w.conv1_b, nullptr, nullptr, n, d.c2, d.c2, 19, 20, 16, 16, 0, ACT_RELU, OP_CORR4};
     layer(l, p);
     if (cls1) {  // conv1_cls + sigmoid (:4733-4741, :4764)
-      p = LayerParams{a3, cls1, packed + g.cls1, w.cls1_b, nullptr, nullptr, n, d.c2, 1, 16, 16, 16, 16, 1, ACT_SIGMOID, OP_CORR3};
+      p = LayerParams{a3, cls1, packed + g.fwd[L_CLS1], w.cls1_b, nullptr, nullptr, n, d.c2, 1, 16, 16, 16, 16, 1, ACT_SIGMOID, OP_CORR3};
       p.out2 = p1;
       l.side_begin();   // auxiliary head: off the critical path
       layer(l, p);
@@ -230,13 +213,13 @@ struct Api {
       return;
     }
     // up2: convT k5 s2 p0 + ReLU (:4712-4719, :4765)
-    p = LayerParams{a3, a4, packed + g.up2, w.up2_b, nullptr, nullptr, n, d.c2, d.c3, 16, 16, 35, 36, 0, ACT_RELU, OP_CONVT};
+    p = LayerParams{a3, a4, packed + g.fwd[L_UP2], w.up2_b, nullptr, nullptr, n, d.c2, d.c3, 16, 16, 35, 36, 0, ACT_RELU, OP_CONVT};
     layer(l, p);
     // conv2: conv k4 + ReLU (:4721-4729, :4766)
-    p = LayerParams{a4, a5, packed + g.conv2, w.conv2_b, nullptr, nullptr, n, d.c3, d.c3, 35, 36, 32, 32, 0, ACT_RELU, OP_CORR4};
+    p = LayerParams{a4, a5, packed + g.fwd[L_CONV2], w.conv2_b, nullptr, nullptr, n, d.c3, d.c3, 35, 36, 32, 32, 0, ACT_RELU, OP_CORR4};
     layer(l, p);
     // conv2_cls + sigmoid (:4731, :4767-4768)
-    p = LayerParams{a5, out, packed + g.cls2, w.cls2_b, nullptr, nullptr, n, d.c3, 1, 32, 32, 32, 32, 1, ACT_SIGMOID, OP_CORR3};
+    p = LayerParams{a5, out, packed + g.fwd[L_CLS2], w.cls2_b, nullptr, nullptr, n, d.c3, 1, 32, 32, 32, 32, 1, ACT_SIGMOID, OP_CORR3};
     p.out2 = p2;
     layer(l, p);
     l.join();
@@ -274,7 +257,7 @@ struct Api {
           forward_layers(l, *desc, *w, packed, latent + b0 * desc->ch * 8, nb, stash, nullptr, nullptr, nullptr, nullptr,
                          nullptr, nullptr, true, sp);   // sp doubles as the padded conv0 output until conv1 is done
           l.pad_conv1(stash + Stash::make(*desc).a3 * nb, sp, (int64_t)nb * desc->c2 * 16);
-          HeadArgs ha{sp, packed + g.up2, packed + g.conv2, packed + g.cls_is, w->up2_b, w->conv2_b, w->cls2_b,
+          HeadArgs ha{sp, packed + g.fwd[L_UP2], packed + g.fwd[L_CONV2], packed + g.cls_is, w->up2_b, w->conv2_b, w->cls2_b,
                       prob_out ? prob_out + b0 * kVox : nullptr, mask + b0 * 1024, counts_out + b0,
                       (float*)(ws + W.off_brow), (float*)(ws + W.off_pl), thh, nb};
           // always one CTA per SM: with fewer (leaf, pass) units than SMs the kernel cuts them along z
@@ -409,7 +392,7 @@ struct Api {
       ChanSumParams c{gl2, gw->cls2_b, n, 1, 32, 32};
       wgrad_bias(l, q, c);
     }
-    p = LayerParams{gl2, g5, packed + g.d_cls2, nullptr, nullptr, a5, n, 1, d.c3, 32, 32, 32, 32, 1, ACT_NONE, OP_CORR3};
+    p = LayerParams{gl2, g5, packed + g.dg[L_CLS2], nullptr, nullptr, a5, n, 1, d.c3, 32, 32, 32, 32, 1, ACT_NONE, OP_CORR3};
     layer(l, p);
     // ---- conv2 ----
     if (wg) {
@@ -417,7 +400,7 @@ struct Api {
       ChanSumParams c{g5, gw->conv2_b, n, d.c3, 32, 32};
       wgrad_bias(l, q, c);
     }
-    p = LayerParams{g5, g4, packed + g.d_conv2, nullptr, nullptr, a4, n, d.c3, d.c3, 32, 32, 35, 36, 3, ACT_NONE, OP_CORR4};
+    p = LayerParams{g5, g4, packed + g.dg[L_CONV2], nullptr, nullptr, a4, n, d.c3, d.c3, 32, 32, 35, 36, 3, ACT_NONE, OP_CORR4};
     layer(l, p);
     // ---- up2 (+ conv1_cls branch) ----
     if (wg) {
@@ -428,9 +411,9 @@ struct Api {
       ChanSumParams c1{gl1, gw->cls1_b, n, 1, 16, 16};
       wgrad_bias(l, q1, c1);
     }
-    p = LayerParams{gl1, tmp3, packed + g.d_cls1, nullptr, nullptr, nullptr, n, 1, d.c2, 16, 16, 16, 16, 1, ACT_NONE, OP_CORR3};
+    p = LayerParams{gl1, tmp3, packed + g.dg[L_CLS1], nullptr, nullptr, nullptr, n, 1, d.c2, 16, 16, 16, 16, 1, ACT_NONE, OP_CORR3};
     layer(l, p);
-    p = LayerParams{g4, g3, packed + g.d_up2, nullptr, tmp3, a3, n, d.c3, d.c2, 35, 36, 16, 16, 0, ACT_NONE, OP_CORR_S2};
+    p = LayerParams{g4, g3, packed + g.dg[L_UP2], nullptr, tmp3, a3, n, d.c3, d.c2, 35, 36, 16, 16, 0, ACT_NONE, OP_CORR_S2};
     layer(l, p);
     // ---- conv1 ----
     if (wg) {
@@ -438,7 +421,7 @@ struct Api {
       ChanSumParams c{g3, gw->conv1_b, n, d.c2, 16, 16};
       wgrad_bias(l, q, c);
     }
-    p = LayerParams{g3, g2, packed + g.d_conv1, nullptr, nullptr, a2, n, d.c2, d.c2, 16, 16, 19, 20, 3, ACT_NONE, OP_CORR4};
+    p = LayerParams{g3, g2, packed + g.dg[L_CONV1], nullptr, nullptr, a2, n, d.c2, d.c2, 16, 16, 19, 20, 3, ACT_NONE, OP_CORR4};
     layer(l, p);
     // ---- up1 (+ conv0_cls branch) ----
     if (wg) {
@@ -449,9 +432,9 @@ struct Api {
       ChanSumParams c0{gl0, gw->cls0_b, n, 1, 8, 8};
       wgrad_bias(l, q0, c0);
     }
-    p = LayerParams{gl0, tmp1, packed + g.d_cls0, nullptr, nullptr, nullptr, n, 1, d.c1, 8, 8, 8, 8, 1, ACT_NONE, OP_CORR3};
+    p = LayerParams{gl0, tmp1, packed + g.dg[L_CLS0], nullptr, nullptr, nullptr, n, 1, d.c1, 8, 8, 8, 8, 1, ACT_NONE, OP_CORR3};
     layer(l, p);
-    p = LayerParams{g2, g1, packed + g.d_up1, nullptr, tmp1, a1, n, d.c2, d.c1, 19, 20, 8, 8, 0, ACT_NONE, OP_CORR_S2};
+    p = LayerParams{g2, g1, packed + g.dg[L_UP1], nullptr, tmp1, a1, n, d.c2, d.c1, 19, 20, 8, 8, 0, ACT_NONE, OP_CORR_S2};
     layer(l, p);
     if (!l.fast_stem_bwd(d, *w, latent, n, x0, a0, g1, gy0, wg ? gw : nullptr, (flags & NVF_BWD_DLATENT) ? g_latent : nullptr)) {
       // ---- conv0 ----
@@ -460,7 +443,7 @@ struct Api {
         ChanSumParams c{g1, gw->conv0_b, n, d.c1, 8, 8};
         wgrad_bias(l, q, c);
       }
-      p = LayerParams{g1, gy0, packed + g.d_conv0, nullptr, nullptr, nullptr, n, d.c1, d.c0, 8, 8, 4, 4, 2, ACT_NONE, OP_CORR_S2};
+      p = LayerParams{g1, gy0, packed + g.dg[L_CONV0], nullptr, nullptr, nullptr, n, d.c1, d.c0, 8, 8, 4, 4, 2, ACT_NONE, OP_CORR_S2};
       layer(l, p);
       // ---- IGDN ----
       {
@@ -476,7 +459,7 @@ struct Api {
         wgrad_bias(l, q, c);
       }
       if (flags & NVF_BWD_DLATENT) {
-        p = LayerParams{gx0, g_latent, packed + g.d_up0, nullptr, nullptr, nullptr, n, d.c0, d.ch, 4, 4, 2, 2, 2, ACT_NONE, OP_CORR_S2};
+        p = LayerParams{gx0, g_latent, packed + g.dg[L_UP0], nullptr, nullptr, nullptr, n, d.c0, d.ch, 4, 4, 2, 2, 2, ACT_NONE, OP_CORR_S2};
         layer(l, p);
       }
     }

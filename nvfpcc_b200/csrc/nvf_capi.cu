@@ -724,27 +724,22 @@ int nvf_train_backward(const NvfDesc* desc, const NvfWeights* w, const float* la
 }
 
 namespace {
-// element counts of the 9 conv kernels / biases in NvfParamSet order
-void conv_sizes(const NvfDesc& d, int (&nw)[NVF_NUM_CONV], int (&nb)[NVF_NUM_CONV]) {
-  const int w[NVF_NUM_CONV] = {d.ch * d.c0 * 125, d.c0 * d.c1 * 125, d.c1 * d.c2 * 125, d.c2 * d.c2 * 64, d.c2 * d.c3 * 125,
-                               d.c3 * d.c3 * 64,  d.c3 * 27,         d.c2 * 27,         d.c1 * 27};
-  const int b[NVF_NUM_CONV] = {d.c0, d.c1, d.c2, d.c2, d.c3, d.c3, 1, 1, 1};
-  for (int i = 0; i < NVF_NUM_CONV; ++i) { nw[i] = w[i]; nb[i] = b[i]; }
-}
+// The job of each layer from its geometry and raw tensors; the callers add the gradient inputs, the outputs and the
+// packed layouts.
 int fill_param_jobs(const NvfDesc& d, const NvfParamSet& ps, fast::ParamPrepParams& pp) {
-  int nw[NVF_NUM_CONV], nb[NVF_NUM_CONV];
-  conv_sizes(d, nw, nb);
   int chunk = 0, noise0 = 0;
   for (int l = 0; l < NVF_NUM_CONV; ++l) {
+    const ConvGeom c = conv_geom(d, l);
     fast::ParamJob& J = pp.job[l];
     if (!ps.kernel[l] || !ps.kernel_init[l] || !ps.b[l] || !ps.b_init[l]) return NVF_ERR_INVALID_ARG;
     J.kernel = ps.kernel[l]; J.init = ps.kernel_init[l]; J.b = ps.b[l]; J.b_init = ps.b_init[l];
-    J.n = nw[l]; J.nb = nb[l];
+    J.n = (int32_t)c.n(); J.nb = c.nb;
     J.chunk0 = chunk;
-    J.nchunks = (nw[l] + fast::kParamChunk - 1) / fast::kParamChunk;
+    J.nchunks = (J.n + fast::kParamChunk - 1) / fast::kParamChunk;
     chunk += J.nchunks;
     J.noise0 = noise0;
-    if (l < NVF_NUM_QUANT) noise0 += nw[l];
+    if (l < NVF_NUM_QUANT) noise0 += J.n;
+    J.A = c.A; J.B = c.B; J.K3 = c.K3(); J.convT = c.convT;   // read only when the job also packs (pk_fwd)
   }
   pp.total_chunks = chunk;
   pp.igdn_beta = ps.igdn_beta; pp.igdn_gamma = ps.igdn_gamma;
@@ -753,12 +748,6 @@ int fill_param_jobs(const NvfDesc& d, const NvfParamSet& ps, fast::ParamPrepPara
   if (!ps.igdn_beta || !ps.igdn_gamma || !ps.lik_sigma || !ps.lik_mu) return NVF_ERR_INVALID_ARG;
   if ((size_t)chunk * 3 * sizeof(float) > NVF_PARAM_WS_BYTES) return NVF_ERR_UNSUPPORTED;
   return NVF_OK;
-}
-float* const* eff_slots_w(const NvfWeightGrads& e, float* (&w)[NVF_NUM_CONV], float* (&b)[NVF_NUM_CONV]) {
-  float* ws[NVF_NUM_CONV] = {e.up0_w, e.conv0_w, e.up1_w, e.conv1_w, e.up2_w, e.conv2_w, e.cls2_w, e.cls1_w, e.cls0_w};
-  float* bs[NVF_NUM_CONV] = {e.up0_b, e.conv0_b, e.up1_b, e.conv1_b, e.up2_b, e.conv2_b, e.cls2_b, e.cls1_b, e.cls0_b};
-  for (int i = 0; i < NVF_NUM_CONV; ++i) { w[i] = ws[i]; b[i] = bs[i]; }
-  return nullptr;
 }
 }  // namespace
 
@@ -774,11 +763,11 @@ int nvf_param_prep(const NvfDesc* desc, const NvfParamSet* params, int q, const 
   fast::ParamPrepParams pp{};
   int rc = fill_param_jobs(*desc, *params, pp);
   if (rc != NVF_OK) return rc;
-  float *w[NVF_NUM_CONV], *b[NVF_NUM_CONV];
-  eff_slots_w(*eff, w, b);
+  float* const* e = slots(*eff);
   for (int i = 0; i < NVF_NUM_CONV; ++i) {
-    if (!w[i] || !b[i]) return NVF_ERR_INVALID_ARG;
-    pp.job[i].w_out = w[i]; pp.job[i].b_out = b[i];
+    const int s = conv_geom(*desc, i).slot;
+    if (!e[s] || !e[s + 1]) return NVF_ERR_INVALID_ARG;
+    pp.job[i].w_out = e[s]; pp.job[i].b_out = e[s + 1];
   }
   if (!eff->igdn_beta || !eff->igdn_gamma) return NVF_ERR_INVALID_ARG;
   pp.beta_out = eff->igdn_beta; pp.gamma_out = eff->igdn_gamma;
@@ -803,13 +792,11 @@ int nvf_param_prep_backward(const NvfDesc* desc, const NvfParamSet* params, floa
   fast::ParamPrepParams pp{};
   int rc = fill_param_jobs(*desc, *params, pp);
   if (rc != NVF_OK) return rc;
-  const float* gw[NVF_NUM_CONV] = {g_eff->up0_w, g_eff->conv0_w, g_eff->up1_w, g_eff->conv1_w, g_eff->up2_w,
-                                   g_eff->conv2_w, g_eff->cls2_w, g_eff->cls1_w, g_eff->cls0_w};
-  const float* gb[NVF_NUM_CONV] = {g_eff->up0_b, g_eff->conv0_b, g_eff->up1_b, g_eff->conv1_b, g_eff->up2_b,
-                                   g_eff->conv2_b, g_eff->cls2_b, g_eff->cls1_b, g_eff->cls0_b};
+  const float* const* ge = slots(*g_eff);
   for (int i = 0; i < NVF_NUM_CONV; ++i) {
-    if (!gw[i] || !gb[i] || !out->kernel[i] || !out->b[i]) return NVF_ERR_INVALID_ARG;
-    pp.job[i].g_w = gw[i]; pp.job[i].g_b = gb[i];
+    const int s = conv_geom(*desc, i).slot;
+    if (!ge[s] || !ge[s + 1] || !out->kernel[i] || !out->b[i]) return NVF_ERR_INVALID_ARG;
+    pp.job[i].g_w = ge[s]; pp.job[i].g_b = ge[s + 1];
     pp.job[i].w_out = out->kernel[i]; pp.job[i].b_out = out->b[i];
   }
   if (!g_eff->igdn_beta || !g_eff->igdn_gamma || !out->igdn_beta || !out->igdn_gamma || !out->lik_sigma || !out->lik_mu)
@@ -831,13 +818,20 @@ int nvf_param_prep_backward(const NvfDesc* desc, const NvfParamSet* params, floa
 
 namespace {
 template <int CH>
-int latent_launch(DevLauncher& l, fast::LatentKParams& kp, bool bwd) {
+void launch_latent(DevLauncher& l, const fast::LatentKParams& kp, bool bwd) {
   int grid = (int)(((int64_t)kp.n * 8 + fast::kLatentThreads - 1) / fast::kLatentThreads);
   if (grid > fast::kLatentMaxCtas) grid = fast::kLatentMaxCtas;
   if (bwd) nvf_launch(fast::k_latent_bwd<CH>, dim3(grid), dim3(fast::kLatentThreads), (size_t)(0), l.st, kp);
   else nvf_launch(fast::k_latent_fwd<CH>, dim3(grid), dim3(fast::kLatentThreads), (size_t)(0), l.st, kp);
   l.post();
-  return l.rc;
+}
+void launch_latent(DevLauncher& l, int ch, const fast::LatentKParams& kp, bool bwd) {
+  switch (ch) {
+    case 1: launch_latent<1>(l, kp, bwd); break;
+    case 2: launch_latent<2>(l, kp, bwd); break;
+    case 3: launch_latent<3>(l, kp, bwd); break;
+    default: launch_latent<4>(l, kp, bwd); break;
+  }
 }
 int latent_call(int ch, const NvfLatentParams* ps, const float* emb, const float* noise, float noise_scale, int train,
                 int64_t n, float beta_bound, float gamma_bound, float pedestal, fast::LatentKParams& kp,
@@ -856,12 +850,8 @@ int latent_call(int ch, const NvfLatentParams* ps, const float* emb, const float
   kp.n = (int32_t)n; kp.train = train ? 1 : 0;
   kp.ticket = (unsigned int*)workspace;
   kp.partial = (double*)((char*)workspace + 16);
-  switch (ch) {
-    case 1: return latent_launch<1>(l, kp, bwd);
-    case 2: return latent_launch<2>(l, kp, bwd);
-    case 3: return latent_launch<3>(l, kp, bwd);
-    default: return latent_launch<4>(l, kp, bwd);
-  }
+  launch_latent(l, ch, kp, bwd);
+  return l.rc;
 }
 }  // namespace
 
@@ -1030,23 +1020,21 @@ int nvf_ffma_microbench(int variant, int64_t iters, float* sink, double* flops_o
 // ------------------------------------------------------------------ fused weight-loop step
 namespace {
 
-// element counts of the 20 effective tensors in NvfWeights / NvfWeightGrads field order
-void eff_sizes(const NvfDesc& d, int64_t (&n)[20]) {
-  const int64_t v[20] = {(int64_t)d.ch * d.c0 * 125, d.c0, d.c0, (int64_t)d.c0 * d.c0, (int64_t)d.c0 * d.c1 * 125, d.c1,
-                         (int64_t)d.c1 * d.c2 * 125, d.c2, (int64_t)d.c2 * d.c2 * 64, d.c2, (int64_t)d.c2 * d.c3 * 125, d.c3,
-                         (int64_t)d.c3 * d.c3 * 64, d.c3, (int64_t)d.c3 * 27, 1, (int64_t)d.c2 * 27, 1, (int64_t)d.c1 * 27, 1};
-  for (int i = 0; i < 20; ++i) n[i] = v[i];
-}
-
 struct StepWs {
   size_t off_train, off_eff, off_geff, off_latent, off_glatent, off_scal, off_param, off_latws, off_tickets, off_losspart, total;
-  int64_t eff_off[20], eff_total;
+  int64_t eff_off[kEffTensors], eff_total;   // the effective tensors in NvfWeights field order
   static StepWs make(const NvfDesc& d, int64_t n) {
     StepWs L{};
-    int64_t sz[20];
-    eff_sizes(d, sz);
+    int64_t sz[kEffTensors];
+    sz[offsetof(NvfWeights, igdn_beta) / sizeof(float*)] = d.c0;
+    sz[offsetof(NvfWeights, igdn_gamma) / sizeof(float*)] = (int64_t)d.c0 * d.c0;
+    for (int l = 0; l < NVF_NUM_CONV; ++l) {
+      const ConvGeom c = conv_geom(d, l);
+      sz[c.slot] = c.n();
+      sz[c.slot + 1] = c.nb;
+    }
     int64_t eo = 0;
-    for (int i = 0; i < 20; ++i) { L.eff_off[i] = eo; eo += (sz[i] + 3) / 4 * 4; }
+    for (int i = 0; i < kEffTensors; ++i) { L.eff_off[i] = eo; eo += (sz[i] + 3) / 4 * 4; }
     L.eff_total = eo;
     size_t o = 0;
     auto take = [&](size_t bytes) { size_t r = o; o += align_up(bytes); return r; };
@@ -1064,30 +1052,6 @@ struct StepWs {
     return L;
   }
 };
-
-template <class PtrT>
-void eff_pointers(float* base, const StepWs& W, PtrT& out) {
-  // NvfWeights / NvfWeightGrads are 20 consecutive pointers in field order
-  auto** slots = reinterpret_cast<float**>(&out);
-  for (int i = 0; i < 20; ++i) slots[i] = base + W.eff_off[i];
-}
-
-template <int CH>
-void launch_latent(DevLauncher& l, fast::LatentKParams& kp, bool bwd) {
-  int grid = (int)(((int64_t)kp.n * 8 + fast::kLatentThreads - 1) / fast::kLatentThreads);
-  if (grid > fast::kLatentMaxCtas) grid = fast::kLatentMaxCtas;
-  if (bwd) nvf_launch(fast::k_latent_bwd<CH>, dim3(grid), dim3(fast::kLatentThreads), (size_t)(0), l.st, kp);
-  else nvf_launch(fast::k_latent_fwd<CH>, dim3(grid), dim3(fast::kLatentThreads), (size_t)(0), l.st, kp);
-  l.post();
-}
-void launch_latent_ch(DevLauncher& l, int ch, fast::LatentKParams& kp, bool bwd) {
-  switch (ch) {
-    case 1: launch_latent<1>(l, kp, bwd); break;
-    case 2: launch_latent<2>(l, kp, bwd); break;
-    case 3: launch_latent<3>(l, kp, bwd); break;
-    default: launch_latent<4>(l, kp, bwd); break;
-  }
-}
 
 int train_step_impl(DevLauncher& l, const NvfStepArgs& a, void* workspace, size_t workspace_bytes) {
   const NvfDesc& d = a.desc;
@@ -1117,12 +1081,9 @@ int train_step_impl(DevLauncher& l, const NvfStepArgs& a, void* workspace, size_
 
   NvfWeights w{};
   NvfWeightGrads gw{}, effw{};
-  eff_pointers(eff, W, effw);
-  eff_pointers(geff, W, gw);
-  {
-    float* const* src = reinterpret_cast<float* const*>(&effw);
-    const float** dst = reinterpret_cast<const float**>(&w);
-    for (int i = 0; i < 20; ++i) dst[i] = src[i];
+  for (int i = 0; i < kEffTensors; ++i) {
+    slots(w)[i] = slots(effw)[i] = eff + W.eff_off[i];
+    slots(gw)[i] = geff + W.eff_off[i];
   }
 
   // ---- latent head on the auxiliary stream ...
@@ -1140,30 +1101,20 @@ int train_step_impl(DevLauncher& l, const NvfStepArgs& a, void* workspace, size_
   lk.seed = a.seed; lk.rng_ctr = (a.noise_latent || !a.train_mode) ? nullptr : ctr;
   lk.latent = latent; lk.bits_out = scal;
   l.side_begin();
-  launch_latent_ch(l, d.ch, lk, false);
+  launch_latent(l, d.ch, lk, false);
   l.side_end();
 
   // ---- ... while the parameter kernel writes the effective tensors, their packed layouts and net_bits
   fast::ParamPrepParams pp{};
   int rc = fill_param_jobs(d, a.params, pp);
   if (rc != NVF_OK) return rc;
-  {
-    float *ww[NVF_NUM_CONV], *bb[NVF_NUM_CONV];
-    eff_slots_w(effw, ww, bb);
-    const GenericPacked g = GenericPacked::make(d);
-    float* packed = (float*)(tws + T.off_packed);
-    const int64_t pf[NVF_NUM_CONV] = {g.up0, g.conv0, g.up1, g.conv1, g.up2, g.conv2, g.cls2, g.cls1, g.cls0};
-    const int64_t pd[NVF_NUM_CONV] = {g.d_up0, g.d_conv0, g.d_up1, g.d_conv1, g.d_up2, g.d_conv2, g.d_cls2, g.d_cls1, g.d_cls0};
-    const int A[NVF_NUM_CONV] = {d.ch, d.c0, d.c1, d.c2, d.c2, d.c3, 1, 1, 1};
-    const int B[NVF_NUM_CONV] = {d.c0, d.c1, d.c2, d.c2, d.c3, d.c3, d.c3, d.c2, d.c1};
-    const int K3[NVF_NUM_CONV] = {125, 125, 125, 64, 125, 64, 27, 27, 27};
-    const int CT[NVF_NUM_CONV] = {1, 1, 1, 0, 1, 0, 0, 0, 0};
-    for (int i = 0; i < NVF_NUM_CONV; ++i) {
-      fast::ParamJob& J = pp.job[i];
-      J.w_out = ww[i]; J.b_out = bb[i];
-      J.pk_fwd = packed + pf[i]; J.pk_dg = packed + pd[i];
-      J.A = A[i]; J.B = B[i]; J.K3 = K3[i]; J.convT = CT[i];
-    }
+  const GenericPacked g = GenericPacked::make(d);
+  float* packed = (float*)(tws + T.off_packed);
+  for (int i = 0; i < NVF_NUM_CONV; ++i) {
+    const int s = conv_geom(d, i).slot;
+    fast::ParamJob& J = pp.job[i];
+    J.w_out = slots(effw)[s]; J.b_out = slots(effw)[s + 1];
+    J.pk_fwd = packed + g.fwd[i]; J.pk_dg = packed + g.dg[i];
   }
   pp.beta_out = effw.igdn_beta; pp.gamma_out = effw.igdn_gamma;
   pp.noise = a.noise_kernel; pp.q = a.q;
@@ -1214,7 +1165,7 @@ int train_step_impl(DevLauncher& l, const NvfStepArgs& a, void* workspace, size_
     lk.gk = G.kernel; lk.gb = G.b; lk.gbeta = G.gdn_beta; lk.ggamma = G.gdn_gamma; lk.gsigma = G.sigma; lk.gmu = G.mu;
   }
   l.side_begin();
-  launch_latent_ch(l, d.ch, lk, true);
+  launch_latent(l, d.ch, lk, true);
   if (need_rng) {
     nvf_launch(fast::k_rng_tick, dim3(1), dim3(1), (size_t)(0), l.st, (unsigned long long*)a.rng_counter);
     l.post();
@@ -1222,13 +1173,11 @@ int train_step_impl(DevLauncher& l, const NvfStepArgs& a, void* workspace, size_
   l.side_end();
   if (wg) {
     const NvfParamGrads& O = a.g_params;
-    const float* const* gwp = reinterpret_cast<const float* const*>(&gw);
-    // field order of NvfWeightGrads: up0_w up0_b igdn_beta igdn_gamma conv0_w conv0_b up1_w ... cls0_w cls0_b
-    const int wi[NVF_NUM_CONV] = {0, 4, 6, 8, 10, 12, 14, 16, 18};
     for (int i = 0; i < NVF_NUM_CONV; ++i) {
       if (!O.kernel[i] || !O.b[i]) return NVF_ERR_INVALID_ARG;
+      const int s = conv_geom(d, i).slot;
       fast::ParamJob& J = pp.job[i];
-      J.g_w = gwp[wi[i]]; J.g_b = gwp[wi[i] + 1];
+      J.g_w = slots(gw)[s]; J.g_b = slots(gw)[s + 1];
       J.w_out = O.kernel[i]; J.b_out = O.b[i];
       J.pk_fwd = nullptr; J.pk_dg = nullptr;
     }

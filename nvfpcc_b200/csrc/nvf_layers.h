@@ -5,6 +5,8 @@
 // configurations that have no fused kernel.  Reference maths: SURVEY.md 3.4/3.5
 // (utils/network.py:4758-4768 forward; autograd of the same ops backward).
 #pragma once
+#include <stddef.h>
+#include <type_traits>
 #include "nvf_common.h"
 #include "nvf_tiles.h"
 #include "../../include/nvf_b200.h"
@@ -493,34 +495,68 @@ struct Stash {
   }
 };
 
-// packed weights for the layer-wise path (forward + dgrad layouts), floats
+// The decoder's nine convolutions in NvfParamSet order; the auxiliary heads cls1 and cls0 come last.
+enum ConvLayer { L_UP0, L_CONV0, L_UP1, L_CONV1, L_UP2, L_CONV2, L_CLS2, L_CLS1, L_CLS0 };
+struct ConvGeom {
+  int A, B, K;   // PyTorch weight (A, B, K, K, K): convT (Cin, Cout, ...), conv (Cout, Cin, ...)
+  bool convT;
+  int nb;        // bias length
+  int slot;      // index of the layer's `_w` pointer in NvfWeights / NvfWeightGrads; `_b` is the next one
+  constexpr int K3() const { return K * K * K; }
+  constexpr int64_t n() const { return (int64_t)A * B * K3(); }   // weight elements
+};
+constexpr ConvGeom conv_geom(const NvfDesc& d, int l) {
+  const ConvGeom g[NVF_NUM_CONV] = {
+      // A     B   K  convT    nb  slot
+      {d.ch, d.c0, 5, true, d.c0, 0},     // up0
+      {d.c0, d.c1, 5, true, d.c1, 4},     // conv0 (igdn_beta, igdn_gamma sit in slots 2, 3)
+      {d.c1, d.c2, 5, true, d.c2, 6},     // up1
+      {d.c2, d.c2, 4, false, d.c2, 8},    // conv1
+      {d.c2, d.c3, 5, true, d.c3, 10},    // up2
+      {d.c3, d.c3, 4, false, d.c3, 12},   // conv2
+      {1, d.c3, 3, false, 1, 14},         // cls2 (conv2_cls)
+      {1, d.c2, 3, false, 1, 16},         // cls1 (conv1_cls)
+      {1, d.c1, 3, false, 1, 18},         // cls0 (conv0_cls)
+  };
+  return g[l];
+}
+
+// NvfWeights / NvfWeightGrads as the array of their pointers in field order
+constexpr int kEffTensors = 20;
+template <class W>
+auto slots(W& w) {
+  return reinterpret_cast<std::remove_reference_t<decltype((w.up0_w))>*>(&w);
+}
+static_assert(sizeof(NvfWeights) == kEffTensors * sizeof(float*) && sizeof(NvfWeightGrads) == sizeof(NvfWeights),
+              "NvfWeights / NvfWeightGrads are plain arrays of pointers");
+#define NVF_CHECK_SLOT(l, f)                                                                          \
+  static_assert(offsetof(NvfWeights, f##_w) == conv_geom(NvfDesc{}, l).slot * sizeof(float*) &&      \
+                    offsetof(NvfWeights, f##_b) == offsetof(NvfWeights, f##_w) + sizeof(float*) &&    \
+                    offsetof(NvfWeightGrads, f##_w) == offsetof(NvfWeights, f##_w) &&                 \
+                    offsetof(NvfWeightGrads, f##_b) == offsetof(NvfWeights, f##_b),                   \
+                #f " slot of conv_geom")
+NVF_CHECK_SLOT(L_UP0, up0);
+NVF_CHECK_SLOT(L_CONV0, conv0);
+NVF_CHECK_SLOT(L_UP1, up1);
+NVF_CHECK_SLOT(L_CONV1, conv1);
+NVF_CHECK_SLOT(L_UP2, up2);
+NVF_CHECK_SLOT(L_CONV2, conv2);
+NVF_CHECK_SLOT(L_CLS2, cls2);
+NVF_CHECK_SLOT(L_CLS1, cls1);
+NVF_CHECK_SLOT(L_CLS0, cls0);
+#undef NVF_CHECK_SLOT
+
+// packed weights for the layer-wise path (forward + dgrad layouts of every layer), floats
 struct GenericPacked {
-  int64_t conv0, up1, conv1, up2, conv2, cls2, cls1, cls0;              // forward packs (up0 uses PACK_CONVT_FWD too)
-  int64_t up0, d_up0, d_conv0, d_up1, d_conv1, d_up2, d_conv2, d_cls2, d_cls1, d_cls0;
+  int64_t fwd[NVF_NUM_CONV], dg[NVF_NUM_CONV];   // by ConvLayer
   int64_t cls_is;  // PACK_CLS_IS copy of cls2 for the fused decode head
   int64_t total;
   static GenericPacked make(const NvfDesc& d) {
     GenericPacked g{};
     int64_t o = 0;
     auto take = [&](int64_t n) { int64_t r = o; o += (n + 3) / 4 * 4; return r; };
-    g.up0 = take((int64_t)d.ch * d.c0 * 125);
-    g.conv0 = take((int64_t)d.c0 * d.c1 * 125);
-    g.up1 = take((int64_t)d.c1 * d.c2 * 125);
-    g.conv1 = take((int64_t)d.c2 * d.c2 * 64);
-    g.up2 = take((int64_t)d.c2 * d.c3 * 125);
-    g.conv2 = take((int64_t)d.c3 * d.c3 * 64);
-    g.cls2 = take((int64_t)d.c3 * 27);
-    g.cls1 = take((int64_t)d.c2 * 27);
-    g.cls0 = take((int64_t)d.c1 * 27);
-    g.d_up0 = take((int64_t)d.ch * d.c0 * 125);
-    g.d_conv0 = take((int64_t)d.c0 * d.c1 * 125);
-    g.d_up1 = take((int64_t)d.c1 * d.c2 * 125);
-    g.d_conv1 = take((int64_t)d.c2 * d.c2 * 64);
-    g.d_up2 = take((int64_t)d.c2 * d.c3 * 125);
-    g.d_conv2 = take((int64_t)d.c3 * d.c3 * 64);
-    g.d_cls2 = take((int64_t)d.c3 * 27);
-    g.d_cls1 = take((int64_t)d.c2 * 27);
-    g.d_cls0 = take((int64_t)d.c1 * 27);
+    for (int l = 0; l < NVF_NUM_CONV; ++l) g.fwd[l] = take(conv_geom(d, l).n());
+    for (int l = 0; l < NVF_NUM_CONV; ++l) g.dg[l] = take(conv_geom(d, l).n());
     g.cls_is = take((int64_t)d.c3 * 36);
     g.total = o;
     return g;

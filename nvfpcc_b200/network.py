@@ -27,7 +27,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import ops
+from . import _lib, ops
 
 # ---------------------------------------------------------------------------
 # shared seed stream (the reference reads SEED3.npy from the CWD at import time,
@@ -265,8 +265,6 @@ class CompDecoder(nn.Module):
     decode_points(x, origins, thh, q) -> dict(coords, counts)     (NVFPCC.py:625-638 batched)
     """
 
-    LAYERS = ("up0", "conv0", "up1", "conv1", "up2", "conv2", "conv2_cls", "conv1_cls", "conv0_cls")
-
     def __init__(self, args, param_model, in_channels=4, useIGDN=False, channels=(8, 16, 8, 8)):
         super().__init__()
         global seed_ptr
@@ -298,18 +296,14 @@ class CompDecoder(nn.Module):
     # -- effective tensors handed to the C ABI ---------------------------------
     def effective_weights(self, q: int, aux: bool = True) -> Dict[str, torch.Tensor]:
         w: Dict[str, torch.Tensor] = {}
-        for name, key in (("up0", "up0"), ("conv0", "conv0"), ("up1", "up1"), ("conv1", "conv1"), ("up2", "up2"),
-                          ("conv2", "conv2"), ("conv2_cls", "cls2")):
-            w[key + "_w"], w[key + "_b"] = getattr(self, name).effective(q)
-        if aux:
-            w["cls1_w"], w["cls1_b"] = self.conv1_cls.effective()
-            w["cls0_w"], w["cls0_b"] = self.conv0_cls.effective()
+        for key, name in _lib.CONV_MODULES.items():
+            if aux or key not in ("cls1", "cls0"):
+                w[key + "_w"], w[key + "_b"] = getattr(self, name).effective(q)
         w["igdn_beta"], w["igdn_gamma"] = self.activation.effective()
         return w
 
     def get_q_params(self) -> List[torch.Tensor]:
-        return [self.up0.kernel, self.conv0.kernel, self.up1.kernel, self.conv1.kernel, self.up2.kernel,
-                self.conv2.kernel, self.conv2_cls.kernel]
+        return [getattr(self, name).kernel for name in list(_lib.CONV_MODULES.values())[:_lib.NVF_NUM_QUANT]]
 
     def net_bits(self) -> torch.Tensor:
         return torch.stack([self.likelihood_model(bypass_round16(p)) for p in self.get_q_params()])
@@ -317,8 +311,7 @@ class CompDecoder(nn.Module):
     def raw_tensors(self) -> Dict[str, torch.Tensor]:
         """The trainable tensors + seed buffers the fused parameter kernels read (ops.RAW_FIELDS)."""
         raw: Dict[str, torch.Tensor] = {}
-        for name, key in (("up0", "up0"), ("conv0", "conv0"), ("up1", "up1"), ("conv1", "conv1"), ("up2", "up2"),
-                          ("conv2", "conv2"), ("conv2_cls", "cls2"), ("conv1_cls", "cls1"), ("conv0_cls", "cls0")):
+        for key, name in _lib.CONV_MODULES.items():
             m = getattr(self, name)
             raw[key + "_kernel"], raw[key + "_kernel_init"], raw[key + "_b"], raw[key + "_b_init"] = (
                 m.kernel, m.kernel_init, m.b, m.b_init)

@@ -227,15 +227,12 @@ class _ParamPrepFn(torch.autograd.Function):
         rawd = dict(zip(RAW_FIELDS, raw))
         ch, channels, beta_bound, gamma_bound = ctx.args
         g_eff = {}
-        for k, g, ref in zip(WEIGHT_FIELDS, grads[:-1], [None] * len(WEIGHT_FIELDS)):
-            g_eff[k] = g
-        shapes = _lib.weight_shapes(ch, channels)
+        for k, g in zip(WEIGHT_FIELDS, grads[:-1]):
+            if g is None:   # shaped like its raw tensor: <key>_kernel for <key>_w, the namesake for the others
+                g = torch.zeros_like(rawd[k[:-1] + "kernel" if k.endswith("_w") else k],
+                                     memory_format=torch.contiguous_format)
+            g_eff[k] = g.contiguous()
         dev = rawd["lik_sigma"].device
-        for k in WEIGHT_FIELDS:
-            if g_eff[k] is None:
-                g_eff[k] = torch.zeros(shapes[k], dtype=torch.float32, device=dev)
-            else:
-                g_eff[k] = g_eff[k].contiguous()
         g_bits = grads[-1] if grads[-1] is not None else torch.zeros(_lib.NVF_NUM_QUANT, device=dev)
         out = b.param_prep_backward(b.desc(ch, channels), rawd, beta_bound, gamma_bound, g_eff, g_bits)
         res = []

@@ -258,15 +258,12 @@ class FusedStepCall:
                     self.grads[id(p_)] = g
                     return g
         raw = rec.raw_tensors()
-        for i, name in enumerate(L.CONV_LAYERS):
-            for field in ("kernel", "kernel_init", "b", "b_init"):
-                getattr(a.params, field)[i] = ptr(raw["%s_%s" % (name, field)].detach())
-            if want_wgrad:
+        a.params = L.param_set(raw, lambda t: ptr(t.detach()))
+        if want_wgrad:
+            for i, name in enumerate(L.CONV_LAYERS):
                 a.g_params.kernel[i] = ptr(gdst(raw[name + "_kernel"]))
                 a.g_params.b[i] = ptr(gdst(raw[name + "_b"]))
-        for field in ("igdn_beta", "igdn_gamma", "lik_sigma", "lik_mu"):
-            setattr(a.params, field, ptr(raw[field].detach()))
-            if want_wgrad:
+            for field in ("igdn_beta", "igdn_gamma", "lik_sigma", "lik_mu"):
                 setattr(a.g_params, field, ptr(gdst(raw[field])))
         lraw = net.latent_raw()
         for field in L.LATENT_FIELDS:
