@@ -32,6 +32,7 @@ def _nvcc() -> str:
 def sources():
     deps = [os.path.join(ROOT, "include", "nvf_b200.h")]
     deps += [os.path.join(ROOT, "include", "nvf_prep_b200.h")]
+    deps += [os.path.join(ROOT, "include", "nvf_metrics_b200.h")]
     deps += [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC)) if f.endswith((".h", ".cu", ".cuh", ".cpp", ".inl"))]
     return deps
 

@@ -50,6 +50,20 @@ def _binding():
     return _bound
 
 
+def as_i32(a, what: str, dev: torch.device) -> torch.Tensor:
+    """(n,3) integer voxel coordinates (numpy or torch, integer or integral float) as a contiguous int32 tensor
+    on `dev`; raises ValueError for another shape or a non-integral coordinate."""
+    t = torch.as_tensor(np.ascontiguousarray(a) if isinstance(a, np.ndarray) else a)
+    if t.dim() != 2 or t.shape[1] != 3:
+        raise ValueError("%s must have shape (n,3)" % what)
+    if t.is_floating_point():
+        r = torch.round(t)
+        if not torch.equal(r, t):
+            raise ValueError("%s must be integer voxel coordinates" % what)
+        t = r
+    return t.to(device=dev, dtype=torch.int32).contiguous()
+
+
 def workspace_bytes(max_cells: int) -> int:
     b = _binding()
     out = C.c_size_t(0)
@@ -74,19 +88,8 @@ def build_grids(points, origins, *, max_cells: Optional[int] = None, max_radius:
     dev = torch.device(device) if device is not None else (
         points.device if isinstance(points, torch.Tensor) and points.is_cuda else torch.device("cuda", torch.cuda.current_device()))
 
-    def as_i32(a, what):
-        t = torch.as_tensor(np.ascontiguousarray(a) if isinstance(a, np.ndarray) else a)
-        if t.dim() != 2 or t.shape[1] != 3:
-            raise ValueError("%s must have shape (n,3)" % what)
-        if t.is_floating_point():
-            r = torch.round(t)
-            if not torch.equal(r, t):
-                raise ValueError("%s must be integer voxel coordinates" % what)
-            t = r
-        return t.to(device=dev, dtype=torch.int32).contiguous()
-
-    pts = as_i32(points, "points")
-    org = as_i32(origins, "origins")
+    pts = as_i32(points, "points", dev)
+    org = as_i32(origins, "origins", dev)
     n, npts = int(org.shape[0]), int(pts.shape[0])
     if max_cells is None:                    # distinct (point >> 5) cells of the cloud, counted on the device
         c = (pts.to(torch.int64) >> 5) + (1 << 20)
@@ -156,9 +159,8 @@ _PLY_TYPES = {"char": "i1", "uchar": "u1", "short": "i2", "ushort": "u2", "int":
               "uint32": "u4", "float32": "f4", "float64": "f8"}
 
 
-def read_ply_xyz(path: str) -> np.ndarray:
-    """Vertex x,y,z of an ASCII or binary PLY as float64 (N,3) - what
-    np.asarray(o3d.io.read_point_cloud(path).points) holds (util_get_grids.py:32,40)."""
+def read_ply_vertex(path: str) -> Dict[str, np.ndarray]:
+    """Every scalar vertex property of an ASCII or binary PLY, by name, as float64 arrays of length N."""
     with open(path, "rb") as f:
         if f.readline().strip() != b"ply":
             raise ValueError("%s is not a PLY file" % path)
@@ -183,15 +185,22 @@ def read_ply_xyz(path: str) -> np.ndarray:
             elif tok[0] == "end_header":
                 break
         names = [p[0] for p in props]
-        if not all(a in names for a in "xyz"):
-            raise ValueError("PLY vertex element has no x/y/z")
         if fmt == "ascii":
             rows = np.loadtxt(f, max_rows=n_vertex, ndmin=2, dtype=np.float64)
-            return np.stack([rows[:, names.index(a)] for a in "xyz"], 1)
+            return {nm: rows[:, i] for i, nm in enumerate(names)}
         order = "<" if fmt == "binary_little_endian" else ">"
         dt = np.dtype([(nm, order + ty) for nm, ty in props])
         rec = np.frombuffer(f.read(n_vertex * dt.itemsize), dtype=dt, count=n_vertex)
-        return np.stack([rec[a].astype(np.float64) for a in "xyz"], 1)
+        return {nm: rec[nm].astype(np.float64) for nm in names}
+
+
+def read_ply_xyz(path: str) -> np.ndarray:
+    """Vertex x,y,z of an ASCII or binary PLY as float64 (N,3) - what
+    np.asarray(o3d.io.read_point_cloud(path).points) holds (util_get_grids.py:32,40)."""
+    v = read_ply_vertex(path)
+    if not all(a in v for a in "xyz"):
+        raise ValueError("PLY vertex element has no x/y/z")
+    return np.stack([v[a] for a in "xyz"], 1)
 
 
 def main(argv=None) -> int:
