@@ -142,3 +142,131 @@ def check_train_against_oracle(binding, fx, golden, dev, blocks=None):
     for k, gv in grads.items():
         close(gv, wo[name_map.get(k, k)].grad, "grad " + k)
     return sums
+
+
+# binding field (include/nvf_b200.h NvfWeights) -> key of O.effective_decoder_weights
+ORACLE_NAME = {"cls2_w": "conv2_cls_w", "cls2_b": "conv2_cls_b", "cls1_w": "conv1_cls_w", "cls1_b": "conv1_cls_b",
+               "cls0_w": "conv0_cls_w", "cls0_b": "conv0_cls_b"}
+
+
+class _ConvRecorder:
+    """Stands in for torch.nn.functional inside the oracle module: conv3d / conv_transpose3d / relu run unchanged, and
+    each convolution's input, weight, bias, arguments and output (with retain_grad) are kept, as is the output of a
+    ReLU applied to it, so that the gradients reaching both are available after backward."""
+
+    def __init__(self):
+        import torch.nn.functional as F
+        self._F = F
+        self.calls = []
+        self.relus = []      # ReLU inputs, in call order
+        self.relu_of = {}    # id(convolution output) -> the ReLU's output
+
+    def relu(self, x):
+        y = self._F.relu(x)
+        y.retain_grad()
+        self.relu_of[id(x)] = y
+        self.relus.append(x)
+        return y
+
+    def _rec(self, fn, x, w, b, args):
+        y = fn(x, w, b, *args)
+        y.retain_grad()
+        self.calls.append((fn, x, w, b, args, y))
+        return y
+
+    def conv3d(self, x, w, b=None, *args):
+        return self._rec(self._F.conv3d, x, w, b, args)
+
+    def conv_transpose3d(self, x, w, b=None, *args):
+        return self._rec(self._F.conv_transpose3d, x, w, b, args)
+
+
+# bound on the float32 forward's error in an activation, relative to that activation's forward scale (the same
+# convolution of |input| with |weight|, plus |bias|): see oracle_train64's S_fwd
+FWD_BAND = 1e-5
+
+
+def oracle_train64(sd, latent, gt=None, dist=None, cot=None):
+    """The float64 oracle of nvf_train_forward -> nvf_loss_seeds -> nvf_train_backward, with autograd.
+
+    The loss is the training loss on (gt, dist) or, with `cot` = (g_out, g_cls1, g_cls0), the sum of the three heads'
+    probabilities weighted by those cotangents.  Besides the heads (probabilities and logits), the loss terms, the
+    gradients of the 20 effective tensors (binding names) and d_latent, it returns `S`, the elementwise scale of each
+    gradient: the same weight-gradient operation (autograd of the oracle's own conv / convT) applied to |input| and
+    |output gradient| (bias: the sum of |output gradient|; d_latent: the data gradient of |output gradient| through
+    |weight|).  |gradient| <= S holds exactly, and S adds up over blocks.
+
+    S bounds what rounding in the gradient's own sums does.  A float32 kernel also works from a float32 forward,
+    whose activations are off by up to FWD_BAND of their forward scale F (the same convolution of |input| with
+    |weight|, plus |bias|).  `S_fwd` bounds what that does to a weight or bias gradient, to first order: the
+    weight-gradient operation applied to FWD_BAND * F of the input (F = |input| where the input is not a ReLU of a
+    convolution) and |output gradient|, plus the full terms of the outputs whose ReLU input lies within FWD_BAND * F
+    of zero, which may fall on the other side of the ReLU (taken with the gradient at the ReLU's output).  It
+    dominates the few entries whose S comes from a handful of activations that are themselves the small remainder of
+    a cancelling sum.  A float32 training step is compared against this oracle within tau * S + S_fwd."""
+    from nvfpcc_b200._lib import WEIGHT_FIELDS
+    wo = {k: v.detach().double().requires_grad_(True) for k, v in O.effective_decoder_weights(sd, 2).items()}
+    lat = latent.detach().double().requires_grad_(True)
+    rec = _ConvRecorder()
+    f0, O.F = O.F, rec
+    try:
+        out, cls0, cls1, logit, _ = O.decoder_forward(lat, wo, aux=True)
+    finally:
+        O.F = f0
+    sums = None
+    if cot is None:
+        gt, dist = gt.double(), dist.double()
+        gts = O.gt_pyramid(gt)
+        sums = (O.surf_focal_dense(out, gt, dist, beta=1, alpha=0.9), O.focal_dense(cls0, gts[0], alpha=0.85),
+                O.focal_dense(cls1, gts[1], alpha=0.85))
+        loss = sums[0] + sums[1] + sums[2]
+    else:
+        loss = sum((p * c.double()).sum() for p, c in zip((out, cls1, cls0), cot))
+    loss.backward()
+    by_ptr = {wo[ORACLE_NAME.get(k, k)].data_ptr(): k for k in WEIGHT_FIELDS}
+    S, S_fwd, logits = {}, {}, {}
+    fscale = {}    # id(convolution output) -> its forward scale F
+
+    def wgrad_of_abs(fn, x, w, args, gy):
+        wd = torch.zeros_like(w.detach()).requires_grad_(True)
+        fn(x.detach().abs(), wd, None, *args).backward(gy)
+        return wd.grad
+
+    with torch.enable_grad():
+        for fn, x, w, b, args, y in rec.calls:
+            with torch.no_grad():
+                fscale[id(y)] = fn(x.abs(), w.abs(), b.abs(), *args)
+        relu_in = {id(rec.relu_of[id(y)]): y for y in rec.relus}    # id(ReLU output) -> its input
+        for fn, x, w, b, args, y in rec.calls:
+            gy = y.grad.detach().abs()
+            kw, kb = by_ptr[w.data_ptr()], by_ptr[b.data_ptr()]
+            shape = wo[ORACLE_NAME.get(kw, kw)].shape
+            logits[kw] = y.detach()
+            S[kw] = wgrad_of_abs(fn, x, w, args, gy).reshape(shape)
+            S[kb] = gy.sum(dim=(0, 2, 3, 4))
+            x_scale = fscale[id(relu_in[id(x)])] if id(x) in relu_in else x.detach()
+            S_fwd[kw] = FWD_BAND * wgrad_of_abs(fn, x_scale, w, args, gy).reshape(shape)
+            S_fwd[kb] = torch.zeros_like(S[kb])
+            if id(y) in rec.relu_of:   # outputs that may fall on the other side of the ReLU
+                g_act = rec.relu_of[id(y)].grad.detach().abs() * (y.detach().abs() <= FWD_BAND * fscale[id(y)])
+                S_fwd[kw] = S_fwd[kw] + wgrad_of_abs(fn, x, w, args, g_act).reshape(shape)
+                S_fwd[kb] = S_fwd[kb] + g_act.sum(dim=(0, 2, 3, 4))
+            if x is lat:
+                xd = torch.zeros_like(lat.detach()).requires_grad_(True)
+                fn(xd, w.detach().abs(), None, *args).backward(gy)
+                S["d_latent"] = xd.grad
+    assert set(S) == set(WEIGHT_FIELDS) | {"d_latent"}
+    return dict(out=out.detach(), cls1=cls1.detach(), cls0=cls0.detach(), logit2=logit.detach(),
+                logit1=logits["cls1_w"], logit0=logits["cls0_w"],
+                sums=None if sums is None else [float(s.detach()) for s in sums],
+                grads={k: wo[ORACLE_NAME.get(k, k)].grad.detach() for k in WEIGHT_FIELDS},
+                d_latent=lat.grad.detach(), S=S, S_fwd=S_fwd)
+
+
+def scaled_err(got, ref, S):
+    """max over elements of |got - ref| / S; an element whose scale S is zero must match exactly (else inf)."""
+    err = (got.detach().cpu().double() - ref.detach().cpu().double()).abs()
+    S = S.detach().cpu().double().reshape(err.shape)
+    if bool(((S == 0) & (err > 0)).any()):
+        return float("inf")
+    return float(torch.where(S > 0, err / torch.where(S > 0, S, torch.ones_like(S)), torch.zeros_like(S)).max())

@@ -128,3 +128,37 @@ def test_train_step_q1_A_and_q2_B_match_reference(golden_train2, tag, q):
                                    err_msg=name)
         n += 1
     assert n == 28
+
+
+def test_float64_train_oracle_and_its_gradient_scales(golden_A):
+    """tests/helpers.oracle_train64, the float64 reference of the training kernels: on the golden training leaves its
+    loss terms and gradients agree with the float32 oracle, every gradient entry is bounded by its scale S
+    (|sum x g| <= sum |x| |g|), the float32 oracle lies within 1e-3 * S + S_fwd of it, and both the gradients and S
+    of a batch are the sums of those of its blocks - the property the batch-decomposition tests rely on."""
+    from tests import helpers as H
+    fx = fixture_inputs("A")
+    gt, dist = torch.from_numpy(golden_A["tr_gt"]).float(), torch.from_numpy(golden_A["tr_dist"]).float()
+    latent = torch.round(torch.randn(2, 3, 2, 2, 2, generator=torch.Generator().manual_seed(5)) * 3)
+    r = H.oracle_train64(fx["sd"], latent, gt, dist)
+    wo = {k: v.clone().requires_grad_(True) for k, v in O.effective_decoder_weights(fx["sd"], 2).items()}
+    lat = latent.clone().requires_grad_(True)
+    out, cls0, cls1, logit, _ = O.decoder_forward(lat, wo, aux=True)
+    gts = O.gt_pyramid(gt)
+    terms = (O.surf_focal_dense(out, gt, dist, beta=1, alpha=0.9), O.focal_dense(cls0, gts[0], alpha=0.85),
+             O.focal_dense(cls1, gts[1], alpha=0.85))
+    sum(terms).backward()
+    for a, b in zip(r["sums"], terms):
+        assert a == pytest.approx(b.item(), rel=1e-5)
+    assert torch.allclose(r["logit2"], logit.detach().double(), rtol=1e-5, atol=1e-5)
+    parts = [H.oracle_train64(fx["sd"], latent[b:b + 1], gt[b:b + 1], dist[b:b + 1]) for b in range(2)]
+    for k, g in r["grads"].items():
+        ref = wo[H.ORACLE_NAME.get(k, k)].grad.double()
+        assert float((g - ref).abs().max()) <= 1e-4 * float(ref.abs().max()), k
+        # the float32 oracle is itself a float32 training step: within 1e-3 * S + S_fwd of the float64 one
+        assert H.scaled_err(ref, g, 1e-3 * r["S"][k] + r["S_fwd"][k]) <= 1.0, k
+        S = r["S"][k]
+        assert bool((g.abs() <= S * (1 + 1e-12)).all()), k
+        assert torch.allclose(parts[0]["S"][k] + parts[1]["S"][k], S, rtol=1e-12, atol=0), k
+        assert torch.allclose(parts[0]["grads"][k] + parts[1]["grads"][k], g, rtol=0, atol=1e-12 * float(S.max())), k
+    assert bool((r["d_latent"].abs() <= r["S"]["d_latent"] * (1 + 1e-12)).all())
+    assert torch.allclose(r["d_latent"][:1], parts[0]["d_latent"], rtol=0, atol=1e-12 * float(r["S"]["d_latent"].max()))
