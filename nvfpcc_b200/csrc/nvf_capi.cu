@@ -8,6 +8,7 @@
 
 #include "nvf_api_impl.h"
 #include "nvf_fast_conv.cuh"
+#include "nvf_fast_dgrad4.cuh"
 #include "nvf_fast_convt.cuh"
 #include "nvf_fast_misc.cuh"
 #include "nvf_fast_stem.cuh"
@@ -361,9 +362,7 @@ struct DevLauncher {
 
   template <int K, int CI, int CO, int DIN, int PAD, int XG, int TY, int NZP, int CIC, int MINB, bool TMA = false, int COTP = 0>
   bool conv_s1(const LayerParams& p) {
-    constexpr int XSH = TMA ? (4 - PAD % 4) % 4 : 0;
-    static_assert(XSH <= 1, "TMA tiles support PAD % 4 in {0, 3}");
-    using G = fast::ConvS1Cfg<K, CI, CO, DIN, PAD, XG, TY, NZP, CIC, XSH, COTP>;
+    using G = fast::ConvS1Cfg<K, CI, CO, DIN, PAD, XG, TY, NZP, CIC, COTP>;
     constexpr int SMEM = TMA ? G::SMEM_BYTES_TMA : G::SMEM_BYTES;
     static_assert(SMEM <= 227 * 1024, "conv_s1 smem");
     auto* k = fast::k_conv_s1<K, CI, CO, DIN, PAD, XG, TY, NZP, CIC, MINB, TMA, COTP>;
@@ -376,6 +375,17 @@ struct DevLauncher {
     }
     fast::ConvS1Params q{p.in, p.out, p.out2, p.Wp, p.bias, p.mask, p.n, p.act};
     nvf_launch(k, dim3(p.n * G::TILES_Z * G::TILES_Y), dim3(G::THREADS), (size_t)(SMEM), st, map, q);
+    post();
+    return true;
+  }
+  template <int C, int D, int TZ, int TY, int MINB>
+  bool conv4_dgrad(const LayerParams& p) {
+    using G = fast::Dgrad4Cfg<C, D, TZ, TY>;
+    static_assert(G::SMEM_BYTES <= 227 * 1024, "conv4 dgrad smem");
+    auto* k = fast::k_conv4_dgrad<C, D, TZ, TY, MINB>;
+    if (!smem_attr(k, G::SMEM_BYTES)) return true;
+    fast::Dgrad4Params q{p.in, p.out, p.Wp, p.mask, p.n};
+    nvf_launch(k, dim3(p.n * G::TILES_Z * G::TILES_Y), dim3(G::THREADS), (size_t)(G::SMEM_BYTES), st, q);
     post();
     return true;
   }
@@ -421,17 +431,17 @@ struct DevLauncher {
   bool fast_layer(const LayerParams& p) {
     if (p.n <= 0) return false;
     if (p.op == OP_CORR4 && p.CI == p.CO && !p.add && !p.out2 && p.act != ACT_SIGMOID) {
-      const bool fwd = p.P == 0 && !p.mask, dg = p.P == 3;
+      const bool fwd = p.P == 0 && !p.mask, dg = p.P == 3 && p.mask && !p.bias && p.act == ACT_NONE;
       if (p.CI == 8) {
         if (fwd && p.Din == 35) return conv_s1<4, 8, 8, 35, 0, 8, 16, 2, 2, 2, true>(p);
-        if (dg && p.Din == 32) return conv_s1<4, 8, 8, 32, 3, 9, 12, 2, 2, 2, true>(p);
+        if (dg && p.Din == 32) return conv4_dgrad<8, 32, 1, 7, 4>(p);
         if (fwd && p.Din == 19) return conv_s1<4, 8, 8, 19, 0, 4, 8, 1, 2, 6, true, 4>(p);
-        if (dg && p.Din == 16) return conv_s1<4, 8, 8, 16, 3, 5, 5, 1, 2, 6, true, 4>(p);    // 640 small CTAs: balance over 148 SMs
+        if (dg && p.Din == 16) return conv4_dgrad<8, 16, 1, 5, 5>(p);
       } else if (p.CI == 16) {
         if (fwd && p.Din == 35) return conv_s1<4, 16, 16, 35, 0, 8, 16, 1, 4, 2>(p);
-        if (dg && p.Din == 32) return conv_s1<4, 16, 16, 32, 3, 9, 12, 1, 4, 2>(p);
+        if (dg && p.Din == 32) return conv4_dgrad<16, 32, 3, 7, 1>(p);
         if (fwd && p.Din == 19) return conv_s1<4, 16, 16, 19, 0, 4, 8, 2, 4, 2>(p);
-        if (dg && p.Din == 16) return conv_s1<4, 16, 16, 16, 3, 5, 10, 2, 4, 2>(p);
+        if (dg && p.Din == 16) return conv4_dgrad<16, 16, 2, 5, 2>(p);
       }
       return false;
     }

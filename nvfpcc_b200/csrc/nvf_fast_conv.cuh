@@ -1,10 +1,12 @@
 // Shared-memory tiled, register-blocked FP32 kernels for the k=4 stride-1
-// convolutions of the NVF decoder's training path (conv1 / conv2 and their
-// data gradients; utils/network.py:4702-4729 via F.conv3d, :687).
+// convolutions of the NVF decoder's training path (conv1 / conv2 forward;
+// utils/network.py:4702-4729 via F.conv3d) and the k=3 classifier heads.
+// The k=4 data gradients are in nvf_fast_dgrad4.cuh.
 //
 //   y[co,z,y,x] = sum_ci sum_k in[ci, z+kz-P, y+ky-P, x+kx-P] * Wp[ci][k][co]
 //   forward:  P = 0, Wp = PACK_CONV_FWD,   epilogue  relu(acc + bias)
-//   dgrad:    P = 3, Wp = PACK_CONV_DGRAD, epilogue  acc masked by (act > 0)
+//   cls head: P = 1 (forward, or data gradient with Wp = PACK_CONV_DGRAD and the
+//             epilogue acc masked by (act > 0))
 //
 // CTA tile: (2*NZP) z-slices x TY rows x 4*XG columns x C output channels.
 // Thread tile: 8 output channels x 4 x x 2 z (64 accumulators).  The input tile
@@ -30,10 +32,7 @@ struct ConvS1Params {
   int32_t n, act;     // act: 0 none, 1 relu, 2 sigmoid
 };
 
-// XSH: extra left shift of the staged columns (tile column = ix + PAD + XSH).  The TMA unit needs the
-// innermost start coordinate of a box to be 16-byte aligned (x0 = -(PAD + XSH) must be a multiple of 4:
-// probed on B200, scripts/probe/tma_probe.cu), so the PAD = 3 data-gradient tiles use XSH = 1.
-template <int K, int CI, int C, int DIN, int PAD, int XG, int TY, int NZP, int CIC, int XSH = 0, int COTP = 0>
+template <int K, int CI, int C, int DIN, int PAD, int XG, int TY, int NZP, int CIC, int COTP = 0>
 struct ConvS1Cfg {
   // output channels per thread; COTP > 0 overrides (smaller tiles = more threads for the small layers)
   static constexpr int COT = COTP > 0 ? COTP : (C >= 8 ? 8 : C);
@@ -45,7 +44,7 @@ struct ConvS1Cfg {
   static constexpr int THREADS = (THREADS_USED + 31) / 32 * 32;
   static constexpr int TZ = 2 * NZP;                      // output slices per tile
   static constexpr int TZI = TZ + K - 1, TYI = TY + K - 1;
-  static constexpr int PI = 4 * XG + 4 + (XSH ? 4 : 0);   // input row pitch (x0 .. x0+7(+XSH) readable)
+  static constexpr int PI = 4 * XG + 4;                   // input row pitch (x0 .. x0+7 readable)
   static constexpr int IN_FLOATS = CIC * TZI * TYI * PI;
   static constexpr int W_FLOATS = CIC * K * K * K * C;
   static constexpr int SMEM_BYTES = (IN_FLOATS + W_FLOATS) * 4;
@@ -59,23 +58,15 @@ struct ConvS1Cfg {
 };
 // One staged chunk of CIC input channels: accumulate into the thread's register tile.
 // s_in: [CIC][TZI][TYI][PI] input tile (halo included), s_w: [CIC][K][K][K][C] weights.
-// eight consecutive tile columns starting at r[XSH] (r 16-byte aligned) as broadcast pairs
-template <int XSH>
+// eight consecutive tile columns starting at r (16-byte aligned) as broadcast pairs
 __device__ __forceinline__ void load_row8_p2(const float* r, p2 (&a)[8]) {
   const float4 lo = *reinterpret_cast<const float4*>(r);
   const float4 hi = *reinterpret_cast<const float4*>(r + 4);
-  if constexpr (XSH == 0) {
-    a[0] = p2_bcast(lo.x); a[1] = p2_bcast(lo.y); a[2] = p2_bcast(lo.z); a[3] = p2_bcast(lo.w);
-    a[4] = p2_bcast(hi.x); a[5] = p2_bcast(hi.y); a[6] = p2_bcast(hi.z); a[7] = p2_bcast(hi.w);
-  } else {
-    static_assert(XSH == 0 || XSH == 1, "XSH");
-    const float4 h2 = *reinterpret_cast<const float4*>(r + 8);
-    a[0] = p2_bcast(lo.y); a[1] = p2_bcast(lo.z); a[2] = p2_bcast(lo.w); a[3] = p2_bcast(hi.x);
-    a[4] = p2_bcast(hi.y); a[5] = p2_bcast(hi.z); a[6] = p2_bcast(hi.w); a[7] = p2_bcast(h2.x);
-  }
+  a[0] = p2_bcast(lo.x); a[1] = p2_bcast(lo.y); a[2] = p2_bcast(lo.z); a[3] = p2_bcast(lo.w);
+  a[4] = p2_bcast(hi.x); a[5] = p2_bcast(hi.y); a[6] = p2_bcast(hi.z); a[7] = p2_bcast(hi.w);
 }
 
-template <class G, int K, int C, int CIC, int COT, int CP, bool PAIR, int XSH>
+template <class G, int K, int C, int CIC, int COT, int CP, bool PAIR>
 __device__ __forceinline__ void conv_s1_chunk(const float* __restrict__ s_in, const float* __restrict__ s_w, int zp, int ty,
                                               int xg, int cg, p2 (&acc2)[2][CP][4], float (&acc)[2][COT][4]) {
 #pragma unroll 1
@@ -86,10 +77,10 @@ __device__ __forceinline__ void conv_s1_chunk(const float* __restrict__ s_in, co
       const float* wp = s_w + ((ci * K) * K + ky) * K * C + cg * COT;
       if constexpr (PAIR) {
         p2 a0[8], a1[8];
-        load_row8_p2<XSH>(rowp, a0);
+        load_row8_p2(rowp, a0);
 #pragma unroll
         for (int kz = 0; kz < K; ++kz) {
-          load_row8_p2<XSH>(rowp + (kz + 1) * G::TYI * G::PI, a1);
+          load_row8_p2(rowp + (kz + 1) * G::TYI * G::PI, a1);
 #pragma unroll
           for (int kx = 0; kx < K; ++kx) {
             const float* wk = wp + (kz * K * K + kx) * C;
@@ -158,12 +149,14 @@ __device__ __forceinline__ void conv_s1_chunk(const float* __restrict__ s_in, co
 
 // TMA = true: the input tile is fetched by the TMA unit (cp.async.bulk.tensor.5d, out-of-bounds = conv halo =
 // zero fill) and the weight chunk by a 1-D bulk copy, double buffered behind two mbarriers, so chunk ch+1
-// streams in while the CTA computes on chunk ch.  TMA = false: cooperative register-staged copy (tmap unused).
+// streams in while the CTA computes on chunk ch.  The TMA unit needs the innermost start coordinate of a box
+// to be 16-byte aligned, so TMA tiles take PAD % 4 == 0.  TMA = false: cooperative register-staged copy
+// (tmap unused).
 template <int K, int CI, int C, int DIN, int PAD, int XG, int TY, int NZP, int CIC, int MINB, bool TMA, int COTP = 0>
-__global__ void __launch_bounds__(ConvS1Cfg<K, CI, C, DIN, PAD, XG, TY, NZP, CIC, 0, COTP>::THREADS, MINB)
+__global__ void __launch_bounds__(ConvS1Cfg<K, CI, C, DIN, PAD, XG, TY, NZP, CIC, COTP>::THREADS, MINB)
     k_conv_s1(const __grid_constant__ CUtensorMap tmap, ConvS1Params p) {
-  constexpr int XSH = TMA ? (4 - PAD % 4) % 4 : 0;
-  using G = ConvS1Cfg<K, CI, C, DIN, PAD, XG, TY, NZP, CIC, XSH, COTP>;
+  static_assert(!TMA || PAD % 4 == 0, "TMA box start must be 16-byte aligned");
+  using G = ConvS1Cfg<K, CI, C, DIN, PAD, XG, TY, NZP, CIC, COTP>;
   constexpr int COT = G::COT;
   extern __shared__ __align__(128) float smem[];
   float* s_in = smem;
@@ -213,7 +206,7 @@ __global__ void __launch_bounds__(ConvS1Cfg<K, CI, C, DIN, PAD, XG, TY, NZP, CIC
     auto issue = [&](int ch) {
       float* dst = smem + (ch & 1) * G::STAGE;
       tma::mbar_arrive_expect_tx(bar + (ch & 1), BYTES);
-      tma::load_5d(dst, &tmap, bar + (ch & 1), -(PAD + XSH), y0 - PAD, z0 - PAD, ch * CIC, b);
+      tma::load_5d(dst, &tmap, bar + (ch & 1), -PAD, y0 - PAD, z0 - PAD, ch * CIC, b);
       tma::load_1d(dst + G::IN_AL, p.Wp + (size_t)ch * G::W_FLOATS, (uint32_t)G::W_FLOATS * 4u, bar + (ch & 1));
     };
     if (tid == 0) {
@@ -224,7 +217,7 @@ __global__ void __launch_bounds__(ConvS1Cfg<K, CI, C, DIN, PAD, XG, TY, NZP, CIC
     for (int ch = 0; ch < NCH; ++ch) {
       tma::mbar_wait(bar + (ch & 1), (uint32_t)(ch >> 1) & 1u);
       const float* st = smem + (ch & 1) * G::STAGE;
-      if (active) conv_s1_chunk<G, K, C, CIC, COT, CP, PAIR, XSH>(st, st + G::IN_AL, zp, ty, xg, cg, acc2, acc);
+      if (active) conv_s1_chunk<G, K, C, CIC, COT, CP, PAIR>(st, st + G::IN_AL, zp, ty, xg, cg, acc2, acc);
       if (ch + 2 < NCH) {
         __syncthreads();               // every thread is done reading this stage
         if (tid == 0) issue(ch + 2);
@@ -278,7 +271,7 @@ __global__ void __launch_bounds__(ConvS1Cfg<K, CI, C, DIN, PAD, XG, TY, NZP, CIC
       }
     }
     __syncthreads();
-    if (active) conv_s1_chunk<G, K, C, CIC, COT, CP, PAIR, XSH>(s_in, s_w, zp, ty, xg, cg, acc2, acc);
+    if (active) conv_s1_chunk<G, K, C, CIC, COT, CP, PAIR>(s_in, s_w, zp, ty, xg, cg, acc2, acc);
   }
   }
   if constexpr (PAIR) {
